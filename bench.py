@@ -21,6 +21,10 @@ Contract (see the task brief): `python bench.py --gpus N --steps K --warmup W` p
   cpu_baseline    the reference-equivalent CPU predict path (oracle port) on a bounded sample, rank 0.
 
 `--impl reference` times that CPU path alone on the same workload definition.
+
+`--dump-outputs DIR` writes what the `value` pass returned in its last timed step on rank 0 - logits [B, 2] and labels
+[B] - as DIR/logits.npy and DIR/labels.npy (float32).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -262,12 +266,13 @@ def run_k2(args, eng, D, sampler):
         labels = []
         ev[0].record()
         for i in range(args.steps):
-            labels.append(step_resident(i)[1])
+            last = step_resident(i)
+            labels.append(last[1])
         mine = torch.cat(labels)
         ev[1].record()
         D.all_gather(mine)   # the path's only exchange: final gather of predictions
         ev[2].record()
-        return ev
+        return ev, last
 
     def settle():
         # The board reaches its power cap within a few tenths of a second of this load and then drops from 1 965 MHz to
@@ -308,7 +313,7 @@ def run_k2(args, eng, D, sampler):
     if sampler:
         sampler.mark_start("k2")
     launches0 = eng.launch_count
-    ev = timed_pass()
+    ev, (logits, labels) = timed_pass()
     D.barrier()
     if sampler:
         sampler.mark_end("k2")
@@ -323,7 +328,7 @@ def run_k2(args, eng, D, sampler):
     D.barrier()
     eng.profile_reset()
     eng.profile(True)
-    evp = timed_pass()
+    evp, _ = timed_pass()
     D.barrier()
     prof = eng.profile_read()
     eng.profile(False)
@@ -347,7 +352,7 @@ def run_k2(args, eng, D, sampler):
     D.barrier()
     if sampler:
         sampler.mark_start("k2_steady")
-    evs = timed_pass()
+    evs, _ = timed_pass()
     D.barrier()
     if sampler:
         sampler.mark_end("k2_steady")
@@ -358,7 +363,8 @@ def run_k2(args, eng, D, sampler):
     e2e_pipelined(eng, [(host_batches[i % N_DISTINCT], offsets_p, T, B) for i in range(args.steps)], B)
     e2e_steady_s = time.perf_counter() - t0
     per_rank = D.gather_floats([ms, gather_ms, ms_prof, kernel_sum, e2e_s * 1e3, e2e_sync_s * 1e3, ms_steady, e2e_steady_s * 1e3])
-    return {"B": B, "L": L, "T": T, "prof": prof, "launches": launches, "per_rank": per_rank}
+    return {"B": B, "L": L, "T": T, "prof": prof, "launches": launches, "per_rank": per_rank,
+            "outputs": {"logits": logits, "labels": labels}}
 
 
 def run_k5(args, eng, D, sampler):
@@ -578,7 +584,10 @@ def main():
     ap.add_argument("--preheat", type=float, default=1.5, help="seconds of load before the steady-state passes")
     ap.add_argument("--no-labels", action="store_true", help="skip the label-agreement pass")
     ap.add_argument("--no-cli", action="store_true", help="skip the 2-GPU CLI check (only runs at --gpus 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's logits and labels as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
 
     from chimeralm_b200.config import DEFAULT_CONFIG as cfg
     from chimeralm_b200.weights import make_state_dict
@@ -622,6 +631,11 @@ def main():
     D.close()
     if rank != 0:
         return
+    if args.dump_outputs:
+        out = Path(args.dump_outputs)
+        out.mkdir(parents=True, exist_ok=True)
+        for name, t in k2["outputs"].items():
+            np.save(out / f"{name}.npy", t.cpu().to(torch.float32).numpy())
 
     B, L, T, prof = k2["B"], k2["L"], k2["T"], k2["prof"]
     per_rank = k2["per_rank"]   # [ms, gather_ms, ms_profiled, kernel_sum_ms, e2e_ms] per rank

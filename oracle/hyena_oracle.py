@@ -23,8 +23,9 @@ What is restated, and from where
   reference holds no golden logits, forward test or fixture for it.  Independent
   cross-checks kept in `tests/test_oracle.py`: the FFT long convolution against a
   float64 direct causal sum, parameter counts against the advertised model size, and
-  `fftconv` / the `pos_emb.z` table against the independent implementation of the same
-  lineage in the installed `fla` package (`fla/modules/conv/long_conv.py`).
+  `fftconv` / the `pos_emb.z` table against outputs of the independent implementation of
+  the same lineage in the `fla` package (`fla/modules/conv/long_conv.py`), stored in
+  `tests/golden/fla_long_conv.npz` by `oracle/make_fla_golden.py`.
 """
 
 from __future__ import annotations
