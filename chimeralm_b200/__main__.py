@@ -1,4 +1,4 @@
-"""`chimeralm` command line: `predict`, `filter`, `--version` with the reference's flags
+"""`chimeralm` command line: `predict`, `filter`, `finetune`, `--version` with the reference's flags
 (`chimeralm/__main__.py:248-333`).  Run as `python -m chimeralm_b200 predict in.bam -o out/`.
 
 Differences kept deliberate and small (SURVEY.md N2): the README-documented but unimplemented
@@ -148,6 +148,35 @@ def filter_bam_by_predcition(bam_path: Path, prediction_path: Path, *, index: bo
         if output_path.exists():
             output_path.unlink()
         raise
+
+
+@app.command()
+def finetune(
+    data_path: Path = typer.Argument(..., help="Labelled reads (.fq/.fastq[.gz] or .parquet); ids end in |0 or |1"),
+    ckpt_path: Path = typer.Option(None, "--ckpt", "-c", help="Model to start from (.ckpt/.pt/.safetensors)"),
+    output_path: Path = typer.Option(..., "--output", "-o", help="Tuned checkpoint (.ckpt, Lightning layout)"),
+    epochs: int = typer.Option(3, "--epochs", "-e", help="Passes over the training reads"),
+    lr: float = typer.Option(1e-3, "--lr", help="AdamW learning rate"),
+    batch_size: int = typer.Option(32, "--batch-size", "-b", help="Reads per batch (batches are bucketed by length)"),
+    seed: int = typer.Option(0, "--seed", help="Seed of the batch order and the dropout masks"),
+    seed_weights: int = typer.Option(0, "--seed-weights", help="Seed of random-init weights when no --ckpt is given"),
+    verbose: bool = typer.Option(False, "--verbose", "-v", help="Enable verbose output"),
+):
+    """Fine-tune the classification head on labelled reads with the backbone frozen (single GPU)."""
+    import torch
+
+    from .train import finetune as run_finetune
+
+    set_logging_level(logging.DEBUG if verbose else logging.INFO)
+    if not torch.cuda.is_available():
+        log.error("No CUDA device: the B200-native path has no CPU fallback.")
+        raise typer.Exit(2)
+    if ckpt_path is None:
+        log.info(f"No --ckpt: starting from seeded random-init ChimeraLM weights (seed {seed_weights})")
+    history = run_finetune(data_path, ckpt_path, output_path, epochs=epochs, lr=lr, batch_size=batch_size, seed=seed,
+                           seed_weights=seed_weights)
+    log.info(f"mean loss per epoch: {', '.join(f'{h:.4f}' for h in history)}")
+    log.info(f"Tuned checkpoint saved to {output_path}")
 
 
 @app.command()

@@ -27,6 +27,11 @@ class clm_config(C.Structure):
 POOLING = {"attention": 0, "mean": 1, "max": 2, "cls": 3}
 
 
+class clm_head_train_cfg(C.Structure):
+    _fields_ = [("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float),
+                ("weight_decay", C.c_float), ("dropout", C.c_double), ("seed", C.c_uint)]
+
+
 class ChimeraLMNativeError(RuntimeError):
     def __init__(self, msg, status: int = 0):
         super().__init__(msg)
@@ -88,6 +93,10 @@ _SIGNATURES = {
     "clm_get_filter": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "clm_set_debug_stop": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "clm_debug_copy": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "clm_head_train_begin": (C.c_int, [C.c_void_p, C.POINTER(clm_head_train_cfg)]),
+    "clm_head_train_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "clm_head_grad_copy": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p]),
+    "clm_head_export": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p]),
     "clm_bam_open": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_void_p)]),
     "clm_bam_close": (None, [C.c_void_p]),
     "clm_bam_error": (C.c_char_p, [C.c_void_p]),

@@ -4,6 +4,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstdio>
@@ -30,6 +31,7 @@
 #include "longconv_tc.cuh"
 #include "longconv_tc2.cuh"
 #include "score_pool.cuh"
+#include "head_train.cuh"
 
 using namespace clm;
 
@@ -101,10 +103,12 @@ struct clm_ctx {
   // head / final
   const float *lnf_g, *lnf_b, *emb;
   __nv_bfloat16* att0_w = nullptr;
+  const float* att0_w32 = nullptr;   // attention.0.weight (fp32, as loaded; refreshed by clm_head_train_step)
   CUtensorMap tm_att0;
   // ln_f affine folded into the scorer (consumes the normalised xn emitted by the last block_mlp)
   __nv_bfloat16* att0_wf = nullptr;
   float* att0_bf = nullptr;
+  float* att0_wf32 = nullptr;   // folded scorer weights in fp32 (source of att0_wf)
   CUtensorMap tm_att0f;
   __nv_bfloat16* emb_norm = nullptr;   // [vocab_rows,256] normalised embedding rows (layer-0 LayerNorm input)
   float *ones = nullptr, *zeros = nullptr;
@@ -215,6 +219,25 @@ struct clm_ctx {
   std::vector<void*> owned;  // device allocations freed at destroy
   std::vector<bm::LayerConsts> h_mlp;     // this model's block-tail constants (the __constant__ bank is per DEVICE, see bind_constants)
   std::set<const void*> smem_attr_done;   // kernels whose dynamic-smem limit was raised on THIS device (per context, not per process)
+  // head fine-tuning (clm_head_train_*): everything is allocated by clm_head_train_begin, nothing per step
+  struct HeadTrain {
+    bool on = false;
+    clm_head_train_cfg cfg{};
+    int max_B = 0;
+    uint32_t thr = 0;          // dropout: keep <=> (hash >> 8) >= thr
+    float scale = 1.f;         // 1 / (1 - p)
+    long long calls = 0;       // clm_head_train_step calls so far: the `step` of the dropout hash
+    long long n = 0;           // elements of the flat head buffers
+    float *param = nullptr, *grad = nullptr, *m = nullptr, *v = nullptr;   // fp32 master copy, gradient, AdamW state
+    int* step = nullptr;       // AdamW steps applied (device)
+    float *z0 = nullptr, *z1 = nullptr, *z2 = nullptr;                        // [B,512] pre-activations
+    float *x1 = nullptr, *x2 = nullptr, *x3 = nullptr, *x4 = nullptr;        // [B,512] layer inputs (after dropout)
+    float *logits = nullptr, *dlogits = nullptr, *fwd_logits = nullptr;      // [B,2]
+    float *dA = nullptr, *dB = nullptr, *dC = nullptr, *dpooled = nullptr;  // [B,512] x3, [B,256]
+    float *rd = nullptr, *gdp = nullptr;                                     // [B][4], [B][256]
+    float *part_dw = nullptr, *part_vec = nullptr;                           // score_bwd_kernel partials
+    int n_cta = 0;
+  } ht;
 };
 
 namespace {
@@ -896,10 +919,10 @@ int launch_longconv_tc(clm_ctx* c, int layer, const __half* vx, const __nv_bfloa
 int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 enum ProfCat { PC_ENCODE = 0, PC_EMBED, PC_LN, PC_GEMM_IN, PC_SHORTCONV, PC_LONGCONV, PC_TRANSPOSE, PC_GEMM_OUT,
-               PC_GEMM_FC1, PC_GEMM_FC2, PC_SCORE, PC_POOL, PC_HEAD, PC_BLOCK_MLP, PC_BLOCK_IN, PC_EMBED_IN, PC_COUNT };
+               PC_GEMM_FC1, PC_GEMM_FC2, PC_SCORE, PC_POOL, PC_HEAD, PC_BLOCK_MLP, PC_BLOCK_IN, PC_EMBED_IN, PC_HEAD_TRAIN, PC_COUNT };
 const char* kProfNames[PC_COUNT] = {"encode", "embed", "layernorm", "gemm_in_proj", "shortconv_gate", "longconv",
                                     "transpose", "gemm_out_proj", "gemm_fc1", "gemm_fc2", "gemm_score", "pool",
-                                    "head", "block_mlp", "block_in", "embed_in"};
+                                    "head", "block_mlp", "block_in", "embed_in", "head_train"};
 
 struct ProfScope {
   clm_ctx* c;
@@ -1032,6 +1055,22 @@ int clm_load_tensor(clm_ctx* c, const char* name, const void* data, int dtype, c
   if (rc) return rc;
   CLM_CUDA(c, cudaMemcpy(t.d, data, (size_t)t.numel * sizeof(float), cudaMemcpyHostToDevice));
   c->w[n] = t;
+  return 0;
+}
+
+// What the forward reads of the attention scorer, derived from attention.0.{weight,bias} and ln_f: the bf16 weights of the
+// unfolded path and ln_f's affine folded into the scorer (W0' = W0 diag(g), b0' = b0 + W0 beta) for score_pool_kernel.
+// clm_finalize builds them; clm_head_train_step rebuilds them in place after every optimizer step (same buffers, so the
+// tensor maps stay valid).
+static int refresh_scorer(clm_ctx* c, cudaStream_t st) {
+  const int D = c->cfg.d_model;
+  const long long n = (long long)D * D;
+  f32_to_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(c->att0_w32, c->att0_w, n);
+  CLM_LAUNCH_CHECK(c, "f32_to_bf16");
+  fold_ln_kernel<<<D, 256, 0, st>>>(c->att0_w32, c->att0_b, c->lnf_g, c->lnf_b, c->att0_wf32, c->att0_bf, D);
+  CLM_LAUNCH_CHECK(c, "fold_ln_f");
+  f32_to_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(c->att0_wf32, c->att0_wf, n);
+  CLM_LAUNCH_CHECK(c, "f32_to_bf16");
   return 0;
 }
 
@@ -1241,15 +1280,14 @@ int clm_finalize(clm_ctx* c) {
     CLM_CUDA(c, cudaMemset(z, 0, ((size_t)D * D + 2 * D) * sizeof(float)));
     a0w = z; c->att0_b = z + (size_t)D * D; c->att2_w = z + (size_t)D * D + D; c->att2_b = 0.f;
   }
-  if ((rc = to_bf16(c, a0w, (int64_t)D * D, &c->att0_w))) return rc;
+  c->att0_w32 = a0w;
+  if ((rc = dev_alloc(c, &c->att0_w, (size_t)D * D))) return rc;
+  if ((rc = dev_alloc(c, &c->att0_wf32, (size_t)D * D))) return rc;
+  if ((rc = dev_alloc(c, &c->att0_bf, (size_t)D))) return rc;
+  if ((rc = dev_alloc(c, &c->att0_wf, (size_t)D * D))) return rc;
+  if ((rc = refresh_scorer(c, 0))) return rc;
   if ((rc = make_tmap_bf16_2d(c, &c->tm_att0, c->att0_w, D, D, 256))) return rc;
   {
-    float* wf = nullptr;
-    if ((rc = dev_alloc(c, &wf, (size_t)D * D))) return rc;
-    if ((rc = dev_alloc(c, &c->att0_bf, (size_t)D))) return rc;
-    fold_ln_kernel<<<D, 256>>>(a0w, c->att0_b, c->lnf_g, c->lnf_b, wf, c->att0_bf, D);
-    CLM_LAUNCH_CHECK(c, "fold_ln_f");
-    if ((rc = to_bf16(c, wf, (int64_t)D * D, &c->att0_wf))) return rc;
     if ((rc = make_tmap_bf16_2d(c, &c->tm_att0f, c->att0_wf, D, D, 256))) return rc;
     if ((rc = dev_alloc(c, &c->emb_norm, (size_t)g.vocab_rows * D))) return rc;
     embed_norm_table_kernel<<<g.vocab_rows, 32>>>(c->emb, c->emb_norm, g.vocab_rows, g.layer_norm_eps);
@@ -1973,3 +2011,205 @@ int clm_debug_copy(clm_ctx* c, const char* what, void* d_dst, size_t max_bytes, 
 }
 
 }  // extern "C"
+
+// =============================================================================================
+// Head fine-tuning (include/chimeralm_b200.h, "Fine-tuning of the head"; csrc/head_train.cuh for the kernels)
+namespace {
+
+// The head tensors in the order of the flat master / gradient / AdamW buffers (offsets rounded up to 64 floats).
+struct HeadTensorInfo { const char* name; long long numel; };
+constexpr HeadTensorInfo kHeadTensors[] = {
+    {"attention.0.weight", 256 * 256}, {"attention.0.bias", 256}, {"attention.2.weight", 256}, {"attention.2.bias", 1},
+    {"classifier.0.weight", 512 * 256}, {"classifier.0.bias", 512}, {"classifier.3.weight", 512 * 512},
+    {"classifier.3.bias", 512}, {"classifier.6.layers.0.weight", 512 * 512}, {"classifier.6.layers.0.bias", 512},
+    {"classifier.6.layers.3.weight", 512 * 512}, {"classifier.6.layers.3.bias", 512}, {"output_layer.weight", 2 * 512},
+    {"output_layer.bias", 2}};
+constexpr int kNumHeadTensors = (int)(sizeof(kHeadTensors) / sizeof(kHeadTensors[0]));
+enum { HT_A0W, HT_A0B, HT_A2W, HT_A2B, HT_C0W, HT_C0B, HT_C3W, HT_C3B, HT_R0W, HT_R0B, HT_R3W, HT_R3B, HT_OW, HT_OB };
+
+long long head_offset(int i) {
+  long long off = 0;
+  for (int k = 0; k < i; ++k) off += (kHeadTensors[k].numel + 63) / 64 * 64;
+  return off;
+}
+
+int head_index(const char* name) {
+  std::string n(name ? name : "");
+  if (n.rfind("net.", 0) != 0) n = "net." + n;
+  for (int i = 0; i < kNumHeadTensors; ++i)
+    if (n == std::string("net.head.") + kHeadTensors[i].name) return i;
+  return -1;
+}
+
+// the tensor the forward reads (as loaded by clm_load_tensor)
+float* head_live(clm_ctx* c, int i) {
+  auto it = c->w.find(std::string("net.head.") + kHeadTensors[i].name);
+  return it == c->w.end() ? nullptr : it->second.d;
+}
+
+}  // namespace
+
+int clm_head_train_begin(clm_ctx* c, const clm_head_train_cfg* cfg) {
+  if (!c || !cfg) return fail(c, CLM_ERR_INVALID, "clm_head_train_begin: bad argument");
+  if (c->cfg.pooling != 0)
+    return fail(c, CLM_ERR_INVALID, "clm_head_train_begin: only attention pooling can be trained (pooling = %d); ChimeraLM's head "
+                "uses attention pooling (chimeralm/models/lm.py:46-55)", c->cfg.pooling);
+  if (!c->finalized) return fail(c, CLM_ERR_STATE, "clm_head_train_begin before clm_finalize");
+  if (c->max_B <= 0) return fail(c, CLM_ERR_STATE, "clm_head_train_begin before clm_reserve");
+  if (c->ht.on) return fail(c, CLM_ERR_STATE, "clm_head_train_begin: training state already exists on this context");
+  if (!(cfg->dropout >= 0.0 && cfg->dropout < 1.0) || !(cfg->lr >= 0.f) || !(cfg->eps > 0.f) || !(cfg->beta1 >= 0.f && cfg->beta1 < 1.f) ||
+      !(cfg->beta2 >= 0.f && cfg->beta2 < 1.f) || !(cfg->weight_decay >= 0.f))
+    return fail(c, CLM_ERR_INVALID, "clm_head_train_begin: lr >= 0, 0 <= betas < 1, eps > 0, weight_decay >= 0, 0 <= dropout < 1");
+  for (int i = 0; i < kNumHeadTensors; ++i)
+    if (!head_live(c, i)) return fail(c, CLM_ERR_MISSING, "clm_head_train_begin: weight 'net.head.%s' was not loaded", kHeadTensors[i].name);
+  CLM_CUDA(c, cudaSetDevice(c->device));
+  clm_ctx::HeadTrain& h = c->ht;
+  const int B = c->max_B, H = c->cfg.head_hidden, D = c->cfg.d_model;
+  h.n = head_offset(kNumHeadTensors);
+  int rc;
+  for (float** p : {&h.param, &h.grad, &h.m, &h.v})
+    if ((rc = dev_alloc(c, p, (size_t)h.n))) return rc;
+  if ((rc = dev_alloc(c, &h.step, 1))) return rc;
+  for (float** p : {&h.z0, &h.z1, &h.z2, &h.x1, &h.x2, &h.x3, &h.x4, &h.dA, &h.dB, &h.dC})
+    if ((rc = dev_alloc(c, p, (size_t)B * H))) return rc;
+  for (float** p : {&h.logits, &h.dlogits, &h.fwd_logits})
+    if ((rc = dev_alloc(c, p, (size_t)B * 2))) return rc;
+  if ((rc = dev_alloc(c, &h.dpooled, (size_t)B * D))) return rc;
+  if ((rc = dev_alloc(c, &h.rd, (size_t)B * 4))) return rc;
+  if ((rc = dev_alloc(c, &h.gdp, (size_t)B * D))) return rc;
+  h.n_cta = std::max(2, c->num_sms / 2 * 2);
+  if ((rc = dev_alloc(c, &h.part_dw, (size_t)h.n_cta * 128 * 256))) return rc;
+  if ((rc = dev_alloc(c, &h.part_vec, (size_t)h.n_cta * 3 * 128))) return rc;
+  CLM_CUDA(c, cudaMemset(h.param, 0, (size_t)h.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(h.grad, 0, (size_t)h.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(h.m, 0, (size_t)h.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(h.v, 0, (size_t)h.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(h.step, 0, sizeof(int)));
+  for (int i = 0; i < kNumHeadTensors; ++i)
+    CLM_CUDA(c, cudaMemcpy(h.param + head_offset(i), head_live(c, i), (size_t)kHeadTensors[i].numel * sizeof(float), cudaMemcpyDeviceToDevice));
+  CLM_CUDA(c, cudaDeviceSynchronize());
+  h.cfg = *cfg;
+  h.max_B = B;
+  h.thr = (uint32_t)std::floor(cfg->dropout * 16777216.0 + 0.5);
+  h.scale = (float)(1.0 / (1.0 - cfg->dropout));
+  h.calls = 0;
+  h.on = true;
+  return 0;
+}
+
+int clm_head_train_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int T, const int64_t* d_targets,
+                        float* d_loss_out, void* stream) {
+  if (!c) return CLM_ERR_INVALID;
+  clm_ctx::HeadTrain& h = c->ht;
+  if (!h.on) return fail(c, CLM_ERR_STATE, "clm_head_train_step before clm_head_train_begin");
+  if (!d_ids || !d_targets || B <= 0 || T <= 0) return fail(c, CLM_ERR_INVALID, "clm_head_train_step: bad argument");
+  if (B > h.max_B) return fail(c, CLM_ERR_STATE, "clm_head_train_step: batch of %d reads exceeds the %d sized by clm_head_train_begin", B, h.max_B);
+  // the backward reads what the folded tail leaves behind: XN from the last block, the per-tile softmax partials of
+  // score_pool_kernel and pooled from head_fused_kernel
+  if (!c->fused_mlp || !c->fused_score_pool || !c->fused_head || c->dbg_layer >= 0)
+    return fail(c, CLM_ERR_STATE, "clm_head_train_step needs the fused forward (options fused_mlp, fused_score_pool, fused_head on, no debug stop)");
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = clm_forward(c, d_ids, ids_dtype, B, T, h.fwd_logits, nullptr, st);
+  if (rc) return rc;
+  const int* status = c->d_status_map + (c->fwd_seq & 7);
+  ProfScope ps_(c, PC_HEAD_TRAIN, st);   // everything after the forward: classifier again, backward, AdamW, refresh
+  const int H = c->cfg.head_hidden, D = c->cfg.d_model;
+  const HeadParams& hp = c->head;
+  const DropoutCfg dc{h.cfg.seed, (uint32_t)h.calls, h.thr, h.scale};
+  const unsigned bt = (unsigned)((B + 31) / 32), bx = (unsigned)((B + HT_RB - 1) / HT_RB);
+  float* G[kNumHeadTensors];
+  for (int i = 0; i < kNumHeadTensors; ++i) G[i] = h.grad + head_offset(i);
+  // ---- classifier forward with dropout (classifier.2, classifier.5, classifier.6.layers.2)
+  ht_fwd_kernel<256, 0><<<dim3(H / 8, bt), 256, 0, st>>>(hp.w0, hp.b0, c->pooled, nullptr, h.z0, h.x1, B, H, dc, 0);
+  CLM_LAUNCH_CHECK(c, "ht_fwd");
+  ht_fwd_kernel<512, 0><<<dim3(H / 8, bt), 256, 0, st>>>(hp.w1, hp.b1, h.x1, nullptr, h.z1, h.x2, B, H, dc, 1);
+  CLM_LAUNCH_CHECK(c, "ht_fwd");
+  ht_fwd_kernel<512, 0><<<dim3(H / 8, bt), 256, 0, st>>>(hp.wr0, hp.br0, h.x2, nullptr, h.z2, h.x3, B, H, dc, 2);
+  CLM_LAUNCH_CHECK(c, "ht_fwd");
+  ht_fwd_kernel<512, 1><<<dim3(H / 8, bt), 256, 0, st>>>(hp.wr1, hp.br1, h.x3, h.x2, nullptr, h.x4, B, H, dc, 0);
+  CLM_LAUNCH_CHECK(c, "ht_fwd");
+  ht_fwd_kernel<512, 2><<<dim3(1, bt), 256, 0, st>>>(hp.wo, hp.bo, h.x4, nullptr, nullptr, h.logits, B, 2, dc, 0);
+  CLM_LAUNCH_CHECK(c, "ht_fwd");
+  ht_loss_kernel<<<1, 256, 0, st>>>(h.logits, d_targets, h.dlogits, d_loss_out, B);
+  CLM_LAUNCH_CHECK(c, "ht_loss");
+  // ---- classifier backward: output_layer, ResidualBlock, classifier.3, classifier.0 -> dpooled
+  ht_bwd_w_kernel<<<dim3(2, 2), 256, 0, st>>>(h.dlogits, h.x4, G[HT_OW], G[HT_OB], B, 2, H);
+  CLM_LAUNCH_CHECK(c, "ht_bwd_w");
+  ht_bwd_x_kernel<<<dim3(H / 256, bx), 256, 0, st>>>(hp.wo, h.dlogits, nullptr, nullptr, h.dA, B, 2, H, dc, 0);          // dx4
+  CLM_LAUNCH_CHECK(c, "ht_bwd_x");
+  ht_bwd_w_kernel<<<dim3(H / 256, H), 256, 0, st>>>(h.dA, h.x3, G[HT_R3W], G[HT_R3B], B, H, H);
+  CLM_LAUNCH_CHECK(c, "ht_bwd_w");
+  ht_bwd_x_kernel<<<dim3(H / 256, bx), 256, 0, st>>>(hp.wr1, h.dA, nullptr, h.z2, h.dB, B, H, H, dc, 2);                // dz2
+  CLM_LAUNCH_CHECK(c, "ht_bwd_x");
+  ht_bwd_w_kernel<<<dim3(H / 256, H), 256, 0, st>>>(h.dB, h.x2, G[HT_R0W], G[HT_R0B], B, H, H);
+  CLM_LAUNCH_CHECK(c, "ht_bwd_w");
+  ht_bwd_x_kernel<<<dim3(H / 256, bx), 256, 0, st>>>(hp.wr0, h.dB, h.dA, h.z1, h.dC, B, H, H, dc, 1);                   // dz1 (+ skip)
+  CLM_LAUNCH_CHECK(c, "ht_bwd_x");
+  ht_bwd_w_kernel<<<dim3(H / 256, H), 256, 0, st>>>(h.dC, h.x1, G[HT_C3W], G[HT_C3B], B, H, H);
+  CLM_LAUNCH_CHECK(c, "ht_bwd_w");
+  ht_bwd_x_kernel<<<dim3(H / 256, bx), 256, 0, st>>>(hp.w1, h.dC, nullptr, h.z0, h.dA, B, H, H, dc, 0);                 // dz0
+  CLM_LAUNCH_CHECK(c, "ht_bwd_x");
+  ht_bwd_w_kernel<<<dim3(D / 256, H), 256, 0, st>>>(h.dA, c->pooled, G[HT_C0W], G[HT_C0B], B, H, D);
+  CLM_LAUNCH_CHECK(c, "ht_bwd_w");
+  ht_bwd_x_kernel<<<dim3(D / 256, bx), 256, 0, st>>>(hp.w0, h.dA, nullptr, nullptr, h.dpooled, B, H, D, dc, 0);         // dpooled
+  CLM_LAUNCH_CHECK(c, "ht_bwd_x");
+  // ---- pooling + scorer backward
+  const int tiles_per_seq = (T + sb::BM - 1) / sb::BM;
+  ht_pool_prep_kernel<<<B, 256, 0, st>>>(c->part, tiles_per_seq, c->pooled, h.dpooled, c->lnf_g, c->lnf_b, h.rd, h.gdp);
+  CLM_LAUNCH_CHECK(c, "ht_pool_prep");
+  {
+    if (int rc_attr = ensure_smem_attr(c, (const void*)(score_bwd_kernel), (int)(sb::SMEM_TOTAL))) return rc_attr;
+    CUtensorMap tmX, tmW;
+    if ((rc = make_tmap_xn(c, &tmX, c->XN, B, T, sb::BM))) return rc;
+    if ((rc = make_tmap_bf16_2d(c, &tmW, c->att0_wf, D, D, sb::HALF))) return rc;   // the forward's folded weights, half a box
+    ScoreBwdParams sp{};
+    sp.b0f = c->att0_bf; sp.w2 = c->att2_w; sp.score = c->score; sp.rd = h.rd; sp.gdp = h.gdp;
+    sp.part_dw = h.part_dw; sp.part_vec = h.part_vec;
+    sp.B = B; sp.T = T; sp.tiles_per_seq = tiles_per_seq; sp.num_tiles = B * tiles_per_seq;
+    const int grid = 2 * std::min(sp.num_tiles, h.n_cta / 2);
+    score_bwd_kernel<<<grid, sb::THREADS, sb::SMEM_TOTAL, st>>>(tmX, tmW, sp);
+    CLM_LAUNCH_CHECK(c, "score_bwd");
+    score_bwd_reduce_kernel<<<D, 256, 0, st>>>(h.part_dw, h.part_vec, grid, c->lnf_g, c->lnf_b, G[HT_A0W], G[HT_A0B], G[HT_A2W], G[HT_A2B]);
+    CLM_LAUNCH_CHECK(c, "score_bwd_reduce");
+  }
+  // ---- AdamW on the master copies, then refresh what the forward reads
+  AdamWParams ap{};
+  ap.p = h.param; ap.m = h.m; ap.v = h.v; ap.g = h.grad; ap.n = h.n;
+  ap.lr = h.cfg.lr; ap.beta1 = h.cfg.beta1; ap.beta2 = h.cfg.beta2; ap.eps = h.cfg.eps; ap.wd = h.cfg.weight_decay;
+  ap.step = h.step; ap.status = status;
+  adamw_kernel<<<(unsigned)std::min<long long>((h.n + 255) / 256, 4LL * c->num_sms), 256, 0, st>>>(ap);
+  CLM_LAUNCH_CHECK(c, "adamw");
+  adamw_step_kernel<<<1, 1, 0, st>>>(h.step, status);
+  CLM_LAUNCH_CHECK(c, "adamw_step");
+  for (int i = 0; i < kNumHeadTensors; ++i)
+    CLM_CUDA(c, cudaMemcpyAsync(head_live(c, i), h.param + head_offset(i), (size_t)kHeadTensors[i].numel * sizeof(float),
+                                cudaMemcpyDeviceToDevice, st));
+  if ((rc = refresh_scorer(c, st))) return rc;
+  ++h.calls;
+  return 0;
+}
+
+int clm_head_grad_copy(clm_ctx* c, const char* name, float* d_dst, void* stream) {
+  if (!c || !name || !d_dst) return fail(c, CLM_ERR_INVALID, "clm_head_grad_copy: bad argument");
+  if (!c->ht.on) return fail(c, CLM_ERR_STATE, "clm_head_grad_copy before clm_head_train_begin");
+  const int i = head_index(name);
+  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_grad_copy: '%s' is not a trainable head tensor", name);
+  CLM_CUDA(c, cudaMemcpyAsync(d_dst, c->ht.grad + head_offset(i), (size_t)kHeadTensors[i].numel * sizeof(float),
+                              cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int clm_head_export(clm_ctx* c, const char* name, float* h_dst) {
+  if (!c || !name || !h_dst) return fail(c, CLM_ERR_INVALID, "clm_head_export: bad argument");
+  if (!c->finalized) return fail(c, CLM_ERR_STATE, "clm_head_export before clm_finalize");
+  const int i = head_index(name);
+  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_export: '%s' is not a head tensor", name);
+  CLM_CUDA(c, cudaSetDevice(c->device));
+  CLM_CUDA(c, cudaDeviceSynchronize());
+  const float* src = c->ht.on ? c->ht.param + head_offset(i) : head_live(c, i);
+  if (!src) return fail(c, CLM_ERR_MISSING, "clm_head_export: weight '%s' was not loaded", name);
+  CLM_CUDA(c, cudaMemcpy(h_dst, src, (size_t)kHeadTensors[i].numel * sizeof(float), cudaMemcpyDeviceToHost));
+  if (c->ht.on)
+    CLM_CUDA(c, cudaMemcpy(&c->att2_b, c->ht.param + head_offset(HT_A2B), sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}

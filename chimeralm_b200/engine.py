@@ -14,8 +14,16 @@ import torch
 
 from . import _lib
 from .config import DEFAULT_CONFIG, HyenaConfig
+from .weights import HEAD_PREFIX
 
 _IDS_DTYPES = {torch.uint8: _lib.CLM_U8, torch.int32: _lib.CLM_I32, torch.int64: _lib.CLM_I64}
+
+
+def _full_name(name: str) -> str:
+    """State-dict key of a head tensor given as "net.head.x", "head.x" or "x"."""
+    if name.startswith("net."):
+        return name
+    return "net." + name if name.startswith("head.") else HEAD_PREFIX + name
 
 
 def _stream_ptr(device) -> C.c_void_p:
@@ -78,9 +86,12 @@ class Engine:
             pass
 
     def load_state_dict(self, sd) -> None:
+        self._head_shapes = getattr(self, "_head_shapes", {})
         for name, t in sd.items():
             if not name.startswith("net."):
                 name = "net." + name
+            if name.startswith(HEAD_PREFIX):
+                self._head_shapes[name] = tuple(t.shape)
             a = t.detach().to(torch.float32).cpu().contiguous().numpy()
             shape = (C.c_int64 * max(a.ndim, 1))(*a.shape) if a.ndim else (C.c_int64 * 1)(1)
             rc = self.lib.clm_load_tensor(self.ctx, name.encode(), a.ctypes.data_as(C.c_void_p), _lib.CLM_F32,
@@ -214,6 +225,72 @@ class Engine:
 
     def predict_host_wait(self, ticket: int) -> None:
         self._check(self.lib.clm_predict_host_wait(self.ctx, int(ticket)), "clm_predict_host_wait")
+
+    # ------------------------------------------------------------------ head fine-tuning (backbone frozen)
+    def head_train_begin(self, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01,
+                         dropout: float = 0.1, seed: int = 0) -> None:
+        """AdamW state and step buffers for batches of up to `max_batch` reads (clm_head_train_begin): the defaults are
+        torch.optim.AdamW's and the reference head's dropout p = 0.1.  Call `reserve` for the largest batch first."""
+        cfg = _lib.clm_head_train_cfg(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay),
+                                      float(dropout), int(seed) & 0xFFFFFFFF)
+        self._check(self.lib.clm_head_train_begin(self.ctx, C.byref(cfg)), "clm_head_train_begin")
+        self.train_steps = 0
+
+    def head_train_step(self, input_ids: torch.Tensor, targets: torch.Tensor, check: bool = True) -> torch.Tensor:
+        """One optimizer step on a batch (clm_head_train_step): ids [B,T] and 0/1 targets [B] -> the batch's mean
+        cross-entropy as a 0-d device tensor.  With `check` the step is synchronised and its status read: an id outside
+        the embedding table raises IndexError; a batch that left the fp16 range of the tensor-core convolution changed
+        no weight and is redone with the fp32 FFT convolution."""
+        if input_ids.dim() != 2 or input_ids.dtype not in _IDS_DTYPES:
+            raise ValueError("input_ids must be [B, T] of uint8/int32/int64")
+        ids = input_ids.to(self.device).contiguous()
+        B, T = ids.shape
+        tgt = torch.as_tensor(targets).to(self.device, torch.int64).contiguous()
+        if tgt.shape != (B,):
+            raise ValueError(f"targets must have shape ({B},), got {tuple(tgt.shape)}")
+        if bool(((tgt != 0) & (tgt != 1)).any()):
+            raise ValueError("targets must be 0 or 1")
+        if T > self.max_tokens or B * T > self.token_budget:
+            raise ValueError(f"batch {B}x{T} exceeds the workspaces reserved before head_train_begin "
+                             f"({self.max_batch} reads, {self.max_tokens} tokens, {self.token_budget} in all)")
+        loss = torch.empty((), dtype=torch.float32, device=self.device)
+        rc = self.lib.clm_head_train_step(self.ctx, C.c_void_p(ids.data_ptr()), _IDS_DTYPES[ids.dtype], B, T,
+                                          C.c_void_p(tgt.data_ptr()), C.c_void_p(loss.data_ptr()), _stream_ptr(self.device))
+        self._check(rc, "clm_head_train_step")
+        self.last_seq = int(self.lib.clm_forward_seq(self.ctx))
+        self.train_steps += 1
+        if check:
+            torch.cuda.current_stream(self.device).synchronize()
+            try:
+                self.forward_status(self.last_seq)
+            except _lib.Fp16RangeError:
+                self.tc_fallbacks += 1
+                self.set_option("tc_conv", 0)
+                try:
+                    return self.head_train_step(ids, tgt, check=True)
+                finally:
+                    self.set_option("tc_conv", 1)
+        return loss
+
+    def head_grad(self, name: str) -> torch.Tensor:
+        """Gradient of head tensor `name` (state-dict key) from the last training step, float32 on this device."""
+        numel = int(np.prod(self._head_shapes[_full_name(name)]))
+        out = torch.empty(numel, dtype=torch.float32, device=self.device)
+        self._check(self.lib.clm_head_grad_copy(self.ctx, _full_name(name).encode(), C.c_void_p(out.data_ptr()),
+                                                _stream_ptr(self.device)), "clm_head_grad_copy")
+        return out.view(self._head_shapes[_full_name(name)])
+
+    def head_export(self, name: str) -> torch.Tensor:
+        """Current value of head tensor `name` as a CPU float32 tensor (synchronises the device)."""
+        shape = self._head_shapes[_full_name(name)]
+        out = torch.empty(shape, dtype=torch.float32)
+        self._check(self.lib.clm_head_export(self.ctx, _full_name(name).encode(), C.c_void_p(out.data_ptr())),
+                    "clm_head_export")
+        return out
+
+    def head_state_dict(self) -> dict:
+        """Every trainable head tensor under its state-dict name."""
+        return {k: self.head_export(k) for k in self._head_shapes}
 
     # ------------------------------------------------------------------ unit-level access (tests)
     def gemm(self, A, W, bias, epi, res=None, w2=None, b2=0.0):

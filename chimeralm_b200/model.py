@@ -18,7 +18,7 @@ from .weights import load_checkpoint, make_state_dict
 
 
 class ClassificationLit:
-    """Inference-only stand-in for the reference LightningModule."""
+    """Stand-in for the reference LightningModule: inference, and training of the head with the backbone frozen."""
 
     def __init__(self, state_dict, *, device: int | str = 0, cfg: HyenaConfig = DEFAULT_CONFIG, max_batch: int = 12,
                  max_tokens: int = 8193, save_attention: bool = False):
@@ -63,6 +63,25 @@ class ClassificationLit:
         return logits
 
     __call__ = forward
+
+    def configure_optimizers(self, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01,
+                             dropout: float = 0.1, seed: int = 0):
+        """AdamW over the head's parameters with the backbone frozen (the reference's configure_optimizers,
+        basic_module.py:200-223, optimises the whole net; here only `net.head.*` is trainable).  Workspaces must already
+        cover the largest training batch (`engine.reserve`)."""
+        self.engine.head_train_begin(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay, dropout=dropout, seed=seed)
+        self._train_begun = True
+        self.training = True
+
+    def training_step(self, batch: dict, batch_idx: int) -> torch.Tensor:
+        """One optimizer step on `batch` (input_ids [B,T], labels [B] of 0/1) and its mean cross-entropy, like the
+        reference's training_step (basic_module.py:87-104, model_step's F.cross_entropy) followed by the optimizer step
+        Lightning takes; returns the loss as a 0-d device tensor."""
+        if not getattr(self, "_train_begun", False):
+            B, T = batch["input_ids"].shape
+            self.engine.reserve(B, T, B * T)
+            self.configure_optimizers()
+        return self.engine.head_train_step(batch["input_ids"], batch["labels"])
 
     def predict_step(self, batch: dict, batch_idx: int):
         """Returns exactly `(logits, batch["labels"])` like the reference (basic_module.py:177-187).  The step is

@@ -205,6 +205,39 @@ int clm_set_debug_stop(clm_ctx* ctx, int layer, int stage);
 /* Copies a named workspace ("resid","xn","u","vx","x0","y","yt","score","pooled") to d_dst. */
 int clm_debug_copy(clm_ctx* ctx, const char* what, void* d_dst, size_t max_bytes, void* stream);
 
+/* ---- Fine-tuning of the head with the backbone frozen ---------------------------------------
+ * Replaces ClassificationLit.training_step / model_step (cross-entropy on net(input_ids),
+ * chimeralm/models/basic_module.py:87-104,106-...) and configure_optimizers (AdamW, :200-223) for the
+ * head's 986 627 parameters (net.head.attention.* and net.head.classifier.* / output_layer.*); the
+ * backbone's weights, filters and spectrum tables are never written.  Attention pooling only (the
+ * named architecture, chimeralm/models/lm.py:46-55): other poolings return CLM_ERR_INVALID.
+ * Without a clm_head_train_begin call the library behaves exactly as without these entry points. */
+typedef struct {
+  float lr, beta1, beta2, eps, weight_decay;   /* torch.optim.AdamW semantics, bias correction included */
+  double dropout;                              /* p of the head's three nn.Dropout layers (0.1 in the reference) */
+  unsigned int seed;                           /* dropout masks: see the hash in csrc/head_train.cuh */
+} clm_head_train_cfg;
+
+/* Allocates the fp32 master copies of the head tensors (initialised from the loaded weights), the AdamW state and every
+ * buffer a step needs, for batches of up to the max_B of the last clm_reserve.  The only allocation: a step allocates
+ * nothing.  Needs clm_finalize and clm_reserve first; a second call returns CLM_ERR_STATE. */
+int clm_head_train_begin(clm_ctx* ctx, const clm_head_train_cfg* cfg);
+/* One optimizer step on a batch: clm_forward with the loaded backbone, the classifier again with dropout, mean cross-
+ * entropy against d_targets (device, int64[B], values 0 / 1), the head's backward and AdamW; afterwards the forward reads
+ * the updated head.  Asynchronous on `stream`; d_loss_out (device float, may be NULL) receives the batch's loss.  The
+ * step's status is that of its forward: clm_forward_status(ctx, clm_forward_seq(ctx)) - and when that is not 0 the step
+ * changed no weight (a batch that left the fp16 range of the tensor-core convolution can be redone with
+ * clm_set_option(ctx, "tc_conv", 0)).  The dropout masks of the k-th call (k = 0, 1, ...) use step = k. */
+int clm_head_train_step(clm_ctx* ctx, const void* d_ids, int ids_dtype, int B, int T, const int64_t* d_targets,
+                        float* d_loss_out, void* stream);
+/* Copies the gradient of head tensor `name` (state-dict key, e.g. "net.head.attention.0.weight") of the last step to the
+ * device buffer d_dst (float32, the tensor's element count).  For parity tests. */
+int clm_head_grad_copy(clm_ctx* ctx, const char* name, float* d_dst, void* stream);
+/* Copies the current value of head tensor `name` to the HOST buffer h_dst (float32).  Synchronises the device.  It also
+ * refreshes the forward's host-side copy of net.head.attention.2.bias, which enters every score of a read equally and so
+ * changes no logit, attention weight or label. */
+int clm_head_export(clm_ctx* ctx, const char* name, float* h_dst);
+
 /* ---- Native BAM ingest (host only, no GPU needed) ----------------------------------------
  * Replaces, for `chimeralm predict`, pysam.AlignmentFile iteration + is_chimeric +
  * parse_bam_file (chimeralm/data/bam.py:21-38) and the per-read Python objects the HF dataset
