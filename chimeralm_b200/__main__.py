@@ -1,4 +1,4 @@
-"""`chimeralm` command line: `predict`, `filter`, `finetune`, `--version` with the reference's flags
+"""`chimeralm` command line: `predict`, `filter`, `finetune`, `evaluate`, `--version` with the reference's flags
 (`chimeralm/__main__.py:248-333`).  Run as `python -m chimeralm_b200 predict in.bam -o out/`.
 
 Differences kept deliberate and small (SURVEY.md N2): the README-documented but unimplemented
@@ -160,6 +160,9 @@ def finetune(
     batch_size: int = typer.Option(32, "--batch-size", "-b", help="Reads per batch (batches are bucketed by length)"),
     seed: int = typer.Option(0, "--seed", help="Seed of the batch order and the dropout masks"),
     seed_weights: int = typer.Option(0, "--seed-weights", help="Seed of random-init weights when no --ckpt is given"),
+    val_path: Path = typer.Option(None, "--val", help="Labelled validation reads: validate every epoch, keep the epoch "
+                                  "with the best F1, write the records to <output>.val.json"),
+    patience: int = typer.Option(None, "--patience", help="With --val: stop after this many epochs without a better F1"),
     verbose: bool = typer.Option(False, "--verbose", "-v", help="Enable verbose output"),
 ):
     """Fine-tune the classification head on labelled reads with the backbone frozen (single GPU)."""
@@ -173,10 +176,59 @@ def finetune(
         raise typer.Exit(2)
     if ckpt_path is None:
         log.info(f"No --ckpt: starting from seeded random-init ChimeraLM weights (seed {seed_weights})")
+    if patience is not None and val_path is None:
+        log.error("--patience needs --val")
+        raise typer.Exit(1)
     history = run_finetune(data_path, ckpt_path, output_path, epochs=epochs, lr=lr, batch_size=batch_size, seed=seed,
-                           seed_weights=seed_weights)
+                           seed_weights=seed_weights, val_path=val_path, patience=patience)
     log.info(f"mean loss per epoch: {', '.join(f'{h:.4f}' for h in history)}")
     log.info(f"Tuned checkpoint saved to {output_path}")
+
+
+@app.command()
+def evaluate(
+    data_path: Path = typer.Argument(..., help="Labelled reads (.fq/.fastq[.gz] or .parquet); ids end in |0 or |1"),
+    ckpt_path: Path = typer.Option(..., "--ckpt", "-c", help="Model to score (.ckpt/.pt/.safetensors)"),
+    batch_size: int = typer.Option(32, "--batch-size", "-b", help="Reads per batch (bucketed by length, as finetune)"),
+    output_path: Path = typer.Option(None, "--output", "-o", help="Write the metrics as JSON"),
+    per_read: Path = typer.Option(None, "--per-read", help="Write name, target, label, p_chimera, loss per read (TSV)"),
+    verbose: bool = typer.Option(False, "--verbose", "-v", help="Enable verbose output"),
+):
+    """Score a model on labelled reads: loss, accuracy, precision, recall, F1, AUROC, confusion matrix (single GPU)."""
+    import json
+
+    import torch
+
+    from .engine import Engine
+    from .train import evaluate as run_evaluate
+    from .train import read_labelled
+    from .weights import load_checkpoint
+
+    set_logging_level(logging.DEBUG if verbose else logging.INFO)
+    try:
+        names, seqs, labels = read_labelled(data_path)
+    except ValueError as e:
+        log.error(str(e))
+        raise typer.Exit(1)
+    if not torch.cuda.is_available():
+        log.error("No CUDA device: the B200-native path has no CPU fallback.")
+        raise typer.Exit(2)
+    eng = Engine(load_checkpoint(ckpt_path), device=0, max_batch=2, max_tokens=1024)   # evaluate() reserves
+    try:
+        metrics, rows = run_evaluate(eng, seqs, labels, batch_size)
+    finally:
+        eng.close()
+    text = json.dumps(metrics)
+    typer.echo(text)
+    if output_path is not None:
+        output_path.parent.mkdir(parents=True, exist_ok=True)
+        output_path.write_text(text + "\n")
+    if per_read is not None:
+        per_read.parent.mkdir(parents=True, exist_ok=True)
+        with per_read.open("w") as f:
+            f.write("name\ttarget\tlabel\tp_chimera\tloss\n")
+            for i, name in enumerate(names):
+                f.write(f"{name}\t{labels[i]}\t{rows['label'][i]}\t{rows['prob'][i]:.9g}\t{rows['loss'][i]:.9g}\n")
 
 
 @app.command()

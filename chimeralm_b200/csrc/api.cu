@@ -919,10 +919,10 @@ int launch_longconv_tc(clm_ctx* c, int layer, const __half* vx, const __nv_bfloa
 int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 enum ProfCat { PC_ENCODE = 0, PC_EMBED, PC_LN, PC_GEMM_IN, PC_SHORTCONV, PC_LONGCONV, PC_TRANSPOSE, PC_GEMM_OUT,
-               PC_GEMM_FC1, PC_GEMM_FC2, PC_SCORE, PC_POOL, PC_HEAD, PC_BLOCK_MLP, PC_BLOCK_IN, PC_EMBED_IN, PC_HEAD_TRAIN, PC_COUNT };
+               PC_GEMM_FC1, PC_GEMM_FC2, PC_SCORE, PC_POOL, PC_HEAD, PC_BLOCK_MLP, PC_BLOCK_IN, PC_EMBED_IN, PC_HEAD_TRAIN, PC_EVAL, PC_COUNT };
 const char* kProfNames[PC_COUNT] = {"encode", "embed", "layernorm", "gemm_in_proj", "shortconv_gate", "longconv",
                                     "transpose", "gemm_out_proj", "gemm_fc1", "gemm_fc2", "gemm_score", "pool",
-                                    "head", "block_mlp", "block_in", "embed_in", "head_train"};
+                                    "head", "block_mlp", "block_in", "embed_in", "head_train", "eval"};
 
 struct ProfScope {
   clm_ctx* c;
@@ -2211,5 +2211,21 @@ int clm_head_export(clm_ctx* c, const char* name, float* h_dst) {
   CLM_CUDA(c, cudaMemcpy(h_dst, src, (size_t)kHeadTensors[i].numel * sizeof(float), cudaMemcpyDeviceToHost));
   if (c->ht.on)
     CLM_CUDA(c, cudaMemcpy(&c->att2_b, c->ht.param + head_offset(HT_A2B), sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// =============================================================================================
+// Evaluation on labelled reads (include/chimeralm_b200.h, "Evaluation"): the forward as predict runs it, then the per-read
+// loss and class-1 probability from its logits (eval_rows_kernel in csrc/head_train.cuh).
+int clm_eval_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int T, const int64_t* d_targets, float* d_logits,
+                  uint8_t* d_labels, float* d_loss, float* d_prob, void* stream) {
+  if (!c) return CLM_ERR_INVALID;
+  if (!d_targets || !d_loss || !d_prob) return fail(c, CLM_ERR_INVALID, "clm_eval_step: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = clm_forward(c, d_ids, ids_dtype, B, T, d_logits, d_labels, st);
+  if (rc) return rc;
+  ProfScope ps_(c, PC_EVAL, st);
+  eval_rows_kernel<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(d_logits, d_targets, d_loss, d_prob, B);
+  CLM_LAUNCH_CHECK(c, "eval_rows");
   return 0;
 }

@@ -87,6 +87,17 @@ __global__ void __launch_bounds__(256) ht_fwd_kernel(const float* __restrict__ W
   }
 }
 
+// Cross-entropy of one read with two classes: lse(l0, l1) - l_y, the max subtracted before the exponentials.  e0, e1 are
+// the shifted exponentials (softmax numerators).  The one definition of the per-read loss: the training step's mean
+// (ht_loss_kernel) and evaluation's per-read values (eval_rows_kernel) are the same numbers.
+struct CeRow { float loss, e0, e1; };
+__device__ __forceinline__ CeRow ce_row(float l0, float l1, int y) {
+  const float m = fmaxf(l0, l1);
+  const float e0 = expf(l0 - m), e1 = expf(l1 - m);
+  const float lse = m + logf(e0 + e1);
+  return {lse - (y ? l1 : l0), e0, e1};
+}
+
 // Mean cross-entropy over the batch (F.cross_entropy, reduction="mean") and its gradient d loss / d logits
 // = (softmax(logits) - onehot(target)) / B.  One block; targets are 0 / 1.
 __global__ void __launch_bounds__(256) ht_loss_kernel(const float* __restrict__ logits, const int64_t* __restrict__ target,
@@ -94,12 +105,10 @@ __global__ void __launch_bounds__(256) ht_loss_kernel(const float* __restrict__ 
   __shared__ float red[8];
   float acc = 0.f;
   for (int b = threadIdx.x; b < B; b += blockDim.x) {
-    const float l0 = logits[2 * b], l1 = logits[2 * b + 1];
-    const float m = fmaxf(l0, l1);
-    const float e0 = expf(l0 - m), e1 = expf(l1 - m);
-    const float lse = m + logf(e0 + e1);
     const int y = target[b] != 0 ? 1 : 0;
-    acc += lse - (y ? l1 : l0);
+    const CeRow r = ce_row(logits[2 * b], logits[2 * b + 1], y);
+    const float e0 = r.e0, e1 = r.e1;
+    acc += r.loss;
     const float inv = 1.0f / (e0 + e1);
     dlogits[2 * b] = (e0 * inv - (y == 0 ? 1.f : 0.f)) / (float)B;
     dlogits[2 * b + 1] = (e1 * inv - (y == 1 ? 1.f : 0.f)) / (float)B;
@@ -112,6 +121,19 @@ __global__ void __launch_bounds__(256) ht_loss_kernel(const float* __restrict__ 
     for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += red[i];
     if (loss_out) *loss_out = t / (float)B;
   }
+}
+
+// Evaluation, per read (ClassificationLit.model_step without the mean and the optimizer step): loss[b] = cross-entropy
+// of logits[b] against target[b] (ce_row, the training loss's arithmetic) and prob[b] = softmax(logits[b])[1], the
+// probability of class 1 (chimera artefact).  prob is formed in fp64 from the fp32 logits, 1 / (1 + exp(l0 - l1)): the
+// difference of the logits is then exact and a small probability keeps its relative precision.  One thread per read.
+__global__ void __launch_bounds__(256) eval_rows_kernel(const float* __restrict__ logits, const int64_t* __restrict__ target,
+                                                        float* __restrict__ loss, float* __restrict__ prob, int B) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const float l0 = logits[2 * b], l1 = logits[2 * b + 1];
+  loss[b] = ce_row(l0, l1, target[b] != 0 ? 1 : 0).loss;
+  prob[b] = (float)(1.0 / (1.0 + exp((double)l0 - (double)l1)));
 }
 
 constexpr int HT_RB = 8;   // reads per block in ht_bwd_x_kernel

@@ -292,6 +292,45 @@ class Engine:
         """Every trainable head tensor under its state-dict name."""
         return {k: self.head_export(k) for k in self._head_shapes}
 
+    # ------------------------------------------------------------------ evaluation on labelled reads
+    def eval_step(self, input_ids: torch.Tensor, targets: torch.Tensor, check: bool = True):
+        """The forward on a labelled batch plus its per-read loss (clm_eval_step): ids [B,T] and 0/1 targets [B] ->
+        (logits float32 [B,2], labels uint8 [B], cross-entropy float32 [B], probability of class 1 float32 [B]), all on
+        this device.  Logits and labels are `forward`'s.  With `check` (as `forward(check=True)`) the call synchronises:
+        an id outside the embedding table raises IndexError, and a batch that left the fp16 range of the tensor-core
+        convolution is redone with the fp32 FFT convolution."""
+        if input_ids.dim() != 2 or input_ids.dtype not in _IDS_DTYPES:
+            raise ValueError("input_ids must be [B, T] of uint8/int32/int64")
+        ids = input_ids.to(self.device).contiguous()
+        B, T = ids.shape
+        tgt = torch.as_tensor(targets).to(self.device, torch.int64).contiguous()
+        if tgt.shape != (B,):
+            raise ValueError(f"targets must have shape ({B},), got {tuple(tgt.shape)}")
+        if bool(((tgt != 0) & (tgt != 1)).any()):
+            raise ValueError("targets must be 0 or 1")
+        self.reserve(B, T, B * T)
+        logits = torch.empty(B, 2, dtype=torch.float32, device=self.device)
+        labels = torch.empty(B, dtype=torch.uint8, device=self.device)
+        loss = torch.empty(B, dtype=torch.float32, device=self.device)
+        prob = torch.empty(B, dtype=torch.float32, device=self.device)
+        rc = self.lib.clm_eval_step(self.ctx, C.c_void_p(ids.data_ptr()), _IDS_DTYPES[ids.dtype], B, T,
+                                    C.c_void_p(tgt.data_ptr()), C.c_void_p(logits.data_ptr()), C.c_void_p(labels.data_ptr()),
+                                    C.c_void_p(loss.data_ptr()), C.c_void_p(prob.data_ptr()), _stream_ptr(self.device))
+        self._check(rc, "clm_eval_step")
+        self.last_seq = int(self.lib.clm_forward_seq(self.ctx))
+        if check:
+            torch.cuda.current_stream(self.device).synchronize()
+            try:
+                self.forward_status(self.last_seq)
+            except _lib.Fp16RangeError:
+                self.tc_fallbacks += 1
+                self.set_option("tc_conv", 0)
+                try:
+                    return self.eval_step(ids, tgt, check=True)
+                finally:
+                    self.set_option("tc_conv", 1)
+        return logits, labels, loss, prob
+
     # ------------------------------------------------------------------ unit-level access (tests)
     def gemm(self, A, W, bias, epi, res=None, w2=None, b2=0.0):
         M, K = A.shape

@@ -83,6 +83,14 @@ class ClassificationLit:
             self.configure_optimizers()
         return self.engine.head_train_step(batch["input_ids"], batch["labels"])
 
+    def validation_step(self, batch: dict, batch_idx: int) -> torch.Tensor:
+        """The reference's validation_step (basic_module.py:87-104, model_step without an optimizer step): the batch's
+        mean cross-entropy as a 0-d device tensor.  Dropout is off and no weight changes.  Synchronous, like `forward`."""
+        _, _, loss, _ = self.engine.eval_step(batch["input_ids"], batch["labels"])
+        return loss.mean()
+
+    test_step = validation_step
+
     def predict_step(self, batch: dict, batch_idx: int):
         """Returns exactly `(logits, batch["labels"])` like the reference (basic_module.py:177-187).  The step is
         asynchronous on the current stream; the device-side argmax labels (same rule as PredictionWriter,

@@ -238,6 +238,21 @@ int clm_head_grad_copy(clm_ctx* ctx, const char* name, float* d_dst, void* strea
  * changes no logit, attention weight or label. */
 int clm_head_export(clm_ctx* ctx, const char* name, float* h_dst);
 
+/* ---- Evaluation on labelled reads ------------------------------------------------------------
+ * Replaces the loss half of ClassificationLit.validation_step / test_step, i.e. model_step without an optimizer step
+ * (cross-entropy on net(input_ids), chimeralm/models/basic_module.py:87-104): clm_forward exactly as above (same logits,
+ * same labels = the head's device argmax), then per read
+ *   d_loss[b] = cross-entropy of d_logits[b] against d_targets[b] (device, int64[B], values 0 / 1), the same per-read
+ *               arithmetic as the mean clm_head_train_step returns (without dropout: the forward applies none);
+ *   d_prob[b] = softmax(d_logits[b])[1], the probability of class 1 (chimera artefact).
+ * d_logits, d_loss, d_prob: device float32 [B,2], [B], [B]; d_labels: device uint8[B] (may be NULL).  Asynchronous on
+ * `stream`, allocates nothing, writes no weight.  Every pooling mode; needs no clm_head_train_begin, and may run between
+ * clm_head_train_step calls on the same context (it then sees the head as trained so far).  Its status is that of its
+ * forward: clm_forward_status(ctx, clm_forward_seq(ctx)); when that is not 0, logits, labels, loss and prob of the batch
+ * are invalid (CLM_ERR_FP16_RANGE: redo it with clm_set_option(ctx, "tc_conv", 0)). */
+int clm_eval_step(clm_ctx* ctx, const void* d_ids, int ids_dtype, int B, int T, const int64_t* d_targets,
+                  float* d_logits, uint8_t* d_labels, float* d_loss, float* d_prob, void* stream);
+
 /* ---- Native BAM ingest (host only, no GPU needed) ----------------------------------------
  * Replaces, for `chimeralm predict`, pysam.AlignmentFile iteration + is_chimeric +
  * parse_bam_file (chimeralm/data/bam.py:21-38) and the per-read Python objects the HF dataset
