@@ -163,14 +163,22 @@ def finetune(
     val_path: Path = typer.Option(None, "--val", help="Labelled validation reads: validate every epoch, keep the epoch "
                                   "with the best F1, write the records to <output>.val.json"),
     patience: int = typer.Option(None, "--patience", help="With --val: stop after this many epochs without a better F1"),
+    train_tail: bool = typer.Option(False, "--train-tail", help="Also train the last block's out_proj, norm2, fc1, fc2 "
+                                    "and ln_f (the rest of the backbone stays frozen)"),
+    tail_lr: float = typer.Option(None, "--tail-lr", help="With --train-tail: AdamW learning rate of those tensors "
+                                  "(default: --lr)"),
     verbose: bool = typer.Option(False, "--verbose", "-v", help="Enable verbose output"),
 ):
-    """Fine-tune the classification head on labelled reads with the backbone frozen (single GPU)."""
+    """Fine-tune the classification head on labelled reads, with the backbone frozen or its last block's tail trained
+    too (single GPU)."""
+    set_logging_level(logging.DEBUG if verbose else logging.INFO)
+    if tail_lr is not None and not train_tail:
+        log.error("--tail-lr needs --train-tail")
+        raise typer.Exit(1)
     import torch
 
     from .train import finetune as run_finetune
 
-    set_logging_level(logging.DEBUG if verbose else logging.INFO)
     if not torch.cuda.is_available():
         log.error("No CUDA device: the B200-native path has no CPU fallback.")
         raise typer.Exit(2)
@@ -180,7 +188,8 @@ def finetune(
         log.error("--patience needs --val")
         raise typer.Exit(1)
     history = run_finetune(data_path, ckpt_path, output_path, epochs=epochs, lr=lr, batch_size=batch_size, seed=seed,
-                           seed_weights=seed_weights, val_path=val_path, patience=patience)
+                           seed_weights=seed_weights, val_path=val_path, patience=patience, train_tail=train_tail,
+                           tail_lr=tail_lr)
     log.info(f"mean loss per epoch: {', '.join(f'{h:.4f}' for h in history)}")
     log.info(f"Tuned checkpoint saved to {output_path}")
 

@@ -97,6 +97,7 @@ _SIGNATURES = {
     "clm_head_train_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "clm_head_grad_copy": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p]),
     "clm_head_export": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p]),
+    "clm_tail_train_begin": (C.c_int, [C.c_void_p, C.c_float]),
     "clm_eval_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_void_p]),
     "clm_bam_open": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_void_p)]),

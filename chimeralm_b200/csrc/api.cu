@@ -32,6 +32,7 @@
 #include "longconv_tc2.cuh"
 #include "score_pool.cuh"
 #include "head_train.cuh"
+#include "tail_train.cuh"
 
 using namespace clm;
 
@@ -48,6 +49,8 @@ struct LayerW {
   const float *in_b, *out_b, *fc1_b, *fc2_b;
   const float *sc_w, *sc_b, *fbias;
   __nv_bfloat16 *in_w, *out_w, *fc1_w, *fc2_w;
+  const float *out_w32, *fc1_w32, *fc2_w32;   // out_proj / fc1 / fc2 weights as loaded (fp32; the tail's trained tensors)
+  float *fc1_wf32 = nullptr, *fc1_bf = nullptr; // fc1 with LayerNorm2 folded in, halved (source of fc1_wt and c_mlp.b1)
   CUtensorMap tm_in, tm_out, tm_fc1, tm_fc2;
   // LayerNorm1 affine folded into in_proj (block_in kernel): W' = W diag(gamma), b' = b + W beta
   __nv_bfloat16* in_wf = nullptr;
@@ -238,6 +241,26 @@ struct clm_ctx {
     float *part_dw = nullptr, *part_vec = nullptr;                           // score_bwd_kernel partials
     int n_cta = 0;
   } ht;
+  // training of the last block's tail together with the head (clm_tail_train_begin): everything is allocated there, for
+  // batches of up to the token budget of the last clm_reserve; nothing per step
+  struct TailTrain {
+    bool on = false;
+    float lr = 0.f;
+    long long n = 0;            // elements of the flat tail buffers
+    long long max_tokens = 0;
+    float *param = nullptr, *grad = nullptr, *m = nullptr, *v = nullptr;   // fp32 master copy, gradient, AdamW state
+    bm::LayerConsts* d_consts = nullptr;   // [n_layer] device copy of h_mlp: the source of the constant bank while training
+    float* R1 = nullptr;                   // r1, then r2 in place (R32 layout)
+    float *rho1 = nullptr, *rho2 = nullptr;                                      // [M]
+    __nv_bfloat16 *n1 = nullptr, *x2 = nullptr, *n2 = nullptr;                   // [M,256]
+    __nv_bfloat16 *h = nullptr, *a = nullptr, *dh = nullptr;                     // [M,d_inner]
+    __nv_bfloat16 *dz = nullptr, *dr2 = nullptr, *dr1 = nullptr;                 // [M,256]
+    __nv_bfloat16 *w0t = nullptr, *w2t = nullptr, *w1t = nullptr;                // per-step transposed weights
+    CUtensorMap tm_w0t, tm_w2t, tm_w1t;
+    float* colsum = nullptr;   // per-warp column partials of the dgrad epilogues
+    float* wpart = nullptr;    // split-K partials of tail_wgrad_kernel
+    long long wpart_elems = 0;
+  } tt;
 };
 
 namespace {
@@ -279,10 +302,14 @@ static const bool g_sync_check = [] { const char* e = getenv("CLM_SYNC_CHECK"); 
 // bm::c_mlp is ONE __constant__ bank per device, shared by every context (model) on it: before a block-tail launch make sure
 // it holds THIS model's biases (a second model finalized on the same device would otherwise silently replace them).
 const clm_ctx* g_const_owner[64] = {nullptr};
+// While the last block's tail is being trained the device copy tt.d_consts is the source (no host round trip per step).
 int bind_constants(clm_ctx* c, cudaStream_t st) {
   const int dev = c->device & 63;
   if (g_const_owner[dev] == c || c->h_mlp.empty()) return 0;
-  CLM_CUDA(c, cudaMemcpyToSymbolAsync(bm::c_mlp, c->h_mlp.data(), c->h_mlp.size() * sizeof(bm::LayerConsts), 0, cudaMemcpyHostToDevice, st));
+  if (c->tt.on)
+    CLM_CUDA(c, cudaMemcpyToSymbolAsync(bm::c_mlp, c->tt.d_consts, c->h_mlp.size() * sizeof(bm::LayerConsts), 0, cudaMemcpyDeviceToDevice, st));
+  else
+    CLM_CUDA(c, cudaMemcpyToSymbolAsync(bm::c_mlp, c->h_mlp.data(), c->h_mlp.size() * sizeof(bm::LayerConsts), 0, cudaMemcpyHostToDevice, st));
   g_const_owner[dev] = c;
   return 0;
 }
@@ -383,11 +410,17 @@ int need(clm_ctx* c, const std::string& name, int64_t numel, const float** out) 
   return 0;
 }
 
-int retile(clm_ctx* c, const float* src, int N, int K, int rt, __nv_bfloat16** out, CUtensorMap* tm) {
-  int rc = dev_alloc(c, out, (size_t)N * K);
-  if (rc) return rc;
-  retile_bf16_kernel<<<(unsigned)(((long long)N * K + 255) / 256), 256>>>(src, *out, N, K, rt);
+// Re-tiles into *out; the first call (*out null) allocates the buffer and encodes its tensor map, later calls rewrite the
+// same buffer on `st`, so the map stays valid.
+int retile(clm_ctx* c, const float* src, int N, int K, int rt, __nv_bfloat16** out, CUtensorMap* tm, cudaStream_t st = 0) {
+  const bool first = *out == nullptr;
+  if (first) {
+    int rc = dev_alloc(c, out, (size_t)N * K);
+    if (rc) return rc;
+  }
+  retile_bf16_kernel<<<(unsigned)(((long long)N * K + 255) / 256), 256, 0, st>>>(src, *out, N, K, rt);
   CLM_LAUNCH_CHECK(c, "retile_bf16");
+  if (!first) return 0;
   cuuint64_t dims[2] = {64, (cuuint64_t)((long long)N * K / 64)};
   cuuint64_t strides[1] = {128};
   cuuint32_t box[2] = {64, 256}, estr[2] = {1, 1};
@@ -410,10 +443,13 @@ int make_tmap_retiled(clm_ctx* c, CUtensorMap* tm, const void* buf, long long ro
   return 0;
 }
 
-int to_bf16(clm_ctx* c, const float* src, int64_t n, __nv_bfloat16** out) {
-  int rc = dev_alloc(c, out, (size_t)n);
-  if (rc) return rc;
-  f32_to_bf16_kernel<<<(unsigned)((n + 255) / 256), 256>>>(src, *out, n);
+// bf16 copy into *out (allocated by the first call, rewritten in place on `st` by later ones)
+int to_bf16(clm_ctx* c, const float* src, int64_t n, __nv_bfloat16** out, cudaStream_t st = 0) {
+  if (!*out) {
+    int rc = dev_alloc(c, out, (size_t)n);
+    if (rc) return rc;
+  }
+  f32_to_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(src, *out, n);
   CLM_LAUNCH_CHECK(c, "f32_to_bf16");
   return 0;
 }
@@ -439,11 +475,18 @@ int launch_gemm(clm_ctx* c, const void* A, const CUtensorMap& tmB, const GemmPar
     if (p.N != 256) return fail(c, CLM_ERR_INVALID, "gemm: scorer epilogue needs N == 256 (got %d)", p.N);
     return launch_gemm_t<256, 2, EPI_SCORE>(c, tmA, tmB, p, st);
   }
+  if (epi == EPI_TAIL_DHID || epi == EPI_TAIL_DR1) {
+    if (p.N != 256) return fail(c, CLM_ERR_INVALID, "gemm: LayerNorm-backward epilogue needs N == 256 (got %d)", p.N);
+    if (epi == EPI_TAIL_DHID) return launch_gemm_t<256, 2, EPI_TAIL_DHID>(c, tmA, tmB, p, st);
+    return launch_gemm_t<256, 2, EPI_TAIL_DR1>(c, tmA, tmB, p, st);
+  }
   if (p.N % 128 != 0) return fail(c, CLM_ERR_INVALID, "gemm: N=%d must be a multiple of 128", p.N);
   switch (epi) {
     case EPI_BIAS_BF16: return launch_gemm_t<128, 3, EPI_BIAS_BF16>(c, tmA, tmB, p, st);
     case EPI_BIAS_GELU_TANH: return launch_gemm_t<128, 3, EPI_BIAS_GELU_TANH>(c, tmA, tmB, p, st);
     case EPI_BIAS_RES_F32: return launch_gemm_t<128, 3, EPI_BIAS_RES_F32>(c, tmA, tmB, p, st);
+    case EPI_BIAS_GELU_TANH_KEEP: return launch_gemm_t<128, 3, EPI_BIAS_GELU_TANH_KEEP>(c, tmA, tmB, p, st);
+    case EPI_TAIL_DH: return launch_gemm_t<128, 3, EPI_TAIL_DH>(c, tmA, tmB, p, st);
     default: return fail(c, CLM_ERR_INVALID, "gemm: unknown epilogue %d", epi);
   }
 }
@@ -1074,6 +1117,45 @@ static int refresh_scorer(clm_ctx* c, cudaStream_t st) {
   return 0;
 }
 
+// What the block tail of layer l reads, derived from its out_proj, norm2, fc1 and fc2 tensors: the bf16 weights of the
+// unfused path, LayerNorm2's affine folded into fc1 (W1' = W1 diag(gamma2), b1' = b1 + W1 beta2), halved because the fused
+// block tail works on h = fc1(x) / 2 (bm::gelu_tanh_bf16x2; exact), and the retiled operands of block_mlp_kernel.  The
+// biases of bm::c_mlp are L.out_b, L.fc2_b and L.fc1_bf.  clm_finalize builds them; with the last block's tail in training
+// clm_head_train_step rebuilds them in place after every optimizer step (same buffers, so the tensor maps stay valid).
+static int prepare_block_tail(clm_ctx* c, int l, cudaStream_t st) {
+  const int D = c->cfg.d_model, DI = c->cfg.d_inner;
+  LayerW& L = c->layers[l];
+  const bool first = L.out_w == nullptr;
+  int rc;
+  if ((rc = to_bf16(c, L.out_w32, (int64_t)D * D, &L.out_w, st))) return rc;
+  if ((rc = to_bf16(c, L.fc1_w32, (int64_t)DI * D, &L.fc1_w, st))) return rc;
+  if ((rc = to_bf16(c, L.fc2_w32, (int64_t)DI * D, &L.fc2_w, st))) return rc;
+  if (first) {
+    if ((rc = make_tmap_bf16_2d(c, &L.tm_out, L.out_w, D, D, 128))) return rc;
+    if ((rc = make_tmap_bf16_2d(c, &L.tm_fc1, L.fc1_w, DI, D, 128))) return rc;
+    if ((rc = make_tmap_bf16_2d(c, &L.tm_fc2, L.fc2_w, D, DI, 128))) return rc;
+    if ((rc = dev_alloc(c, &L.fc1_wf32, (size_t)DI * D))) return rc;
+    if ((rc = dev_alloc(c, &L.fc1_bf, (size_t)DI))) return rc;
+  }
+  fold_ln_kernel<<<DI, 256, 0, st>>>(L.fc1_w32, L.fc1_b, L.ln2_g, L.ln2_b, L.fc1_wf32, L.fc1_bf, D);
+  CLM_LAUNCH_CHECK(c, "fold_ln2");
+  scale_f32_kernel<<<(unsigned)(((size_t)DI * D + 255) / 256), 256, 0, st>>>(L.fc1_wf32, (long long)DI * D, 0.5f);
+  scale_f32_kernel<<<(unsigned)((DI + 255) / 256), 256, 0, st>>>(L.fc1_bf, DI, 0.5f);
+  CLM_LAUNCH_CHECK(c, "scale_fc1");
+  if ((rc = retile(c, L.out_w32, D, D, 256, &L.out_wt, &L.tm_out_t, st))) return rc;
+  if ((rc = retile(c, L.fc1_wf32, DI, D, 128, &L.fc1_wt, &L.tm_fc1_t, st))) return rc;
+  if ((rc = retile(c, L.fc2_w32, D, DI, 256, &L.fc2_wt, &L.tm_fc2_t, st))) return rc;
+#ifdef CLM_EXPERIMENTS
+  if ((rc = retile(c, L.fc1_wf32, DI, D, 64, &L.fc1_w64, &L.tm_fc1_64, st))) return rc;
+  if (first) {
+    if ((rc = make_tmap_retiled(c, &L.tm_out_h, L.out_wt, (long long)D * D / 64, 128))) return rc;
+    if ((rc = make_tmap_retiled(c, &L.tm_fc1_h, L.fc1_wt, (long long)DI * D / 64, 64))) return rc;
+    if ((rc = make_tmap_retiled(c, &L.tm_fc2_h, L.fc2_wt, (long long)DI * D / 64, 128))) return rc;
+  }
+#endif
+  return 0;
+}
+
 // Input scale of the tensor-core convolution, per layer and channel: one small forward (fp32 convolution) over a fixed
 // synthetic draw - a read of random bases and a half-[PAD] read, the two regimes real batches consist of - records
 // max |v * x1|, and tc::scales_kernel turns it into the power-of-two factors block_in / longconv_tc apply.  LayerNorm
@@ -1140,9 +1222,6 @@ int clm_finalize(clm_ctx* c) {
     NEED(P + "mlp.fc2.weight", (int64_t)g.d_inner * D, &fc2_w);
     NEED(P + "mlp.fc2.bias", D, &L.fc2_b);
     if ((rc = to_bf16(c, in_w, 3LL * D * D, &L.in_w))) return rc;
-    if ((rc = to_bf16(c, out_w, (int64_t)D * D, &L.out_w))) return rc;
-    if ((rc = to_bf16(c, fc1_w, (int64_t)g.d_inner * D, &L.fc1_w))) return rc;
-    if ((rc = to_bf16(c, fc2_w, (int64_t)g.d_inner * D, &L.fc2_w))) return rc;
     if ((rc = make_tmap_bf16_2d(c, &L.tm_in, L.in_w, 3 * D, D, 128))) return rc;
     {
       float* wf = nullptr;
@@ -1156,36 +1235,14 @@ int clm_finalize(clm_ctx* c) {
       if ((rc = make_tmap_retiled(c, &L.tm_inf_h, L.in_wf, (long long)3 * D * D / 64, 128))) return rc;
 #endif
     }
-    if ((rc = make_tmap_bf16_2d(c, &L.tm_out, L.out_w, D, D, 128))) return rc;
-    if ((rc = make_tmap_bf16_2d(c, &L.tm_fc1, L.fc1_w, g.d_inner, D, 128))) return rc;
-    if ((rc = make_tmap_bf16_2d(c, &L.tm_fc2, L.fc2_w, D, g.d_inner, 128))) return rc;
-    {
-      if (l >= bm::MAX_LAYERS) return fail(c, CLM_ERR_INVALID, "n_layer > %d not supported by the fused block kernel", bm::MAX_LAYERS);
-      // LayerNorm2 affine folded into fc1: W1' = W1 diag(gamma2), b1' = b1 + W1 beta2
-      float *w1f = nullptr, *b1f = nullptr;
-      if ((rc = dev_alloc(c, &w1f, (size_t)g.d_inner * D))) return rc;
-      if ((rc = dev_alloc(c, &b1f, (size_t)g.d_inner))) return rc;
-      fold_ln_kernel<<<g.d_inner, 256>>>(fc1_w, L.fc1_b, L.ln2_g, L.ln2_b, w1f, b1f, D);
-      CLM_LAUNCH_CHECK(c, "fold_ln2");
-      // the fused block tail works on h = fc1(x) / 2 (bm::gelu_tanh_bf16x2): halve W1' and b1' (exact)
-      scale_f32_kernel<<<(unsigned)(((size_t)g.d_inner * D + 255) / 256), 256>>>(w1f, (long long)g.d_inner * D, 0.5f);
-      scale_f32_kernel<<<(unsigned)((g.d_inner + 255) / 256), 256>>>(b1f, g.d_inner, 0.5f);
-      CLM_LAUNCH_CHECK(c, "scale_fc1");
-      if ((rc = retile(c, out_w, D, D, 256, &L.out_wt, &L.tm_out_t))) return rc;
-      if ((rc = retile(c, w1f, g.d_inner, D, 128, &L.fc1_wt, &L.tm_fc1_t))) return rc;
-      if ((rc = retile(c, fc2_w, D, g.d_inner, 256, &L.fc2_wt, &L.tm_fc2_t))) return rc;
-#ifdef CLM_EXPERIMENTS
-      if ((rc = retile(c, w1f, g.d_inner, D, 64, &L.fc1_w64, &L.tm_fc1_64))) return rc;
-      if ((rc = make_tmap_retiled(c, &L.tm_out_h, L.out_wt, (long long)D * D / 64, 128))) return rc;
-      if ((rc = make_tmap_retiled(c, &L.tm_fc1_h, L.fc1_wt, (long long)g.d_inner * D / 64, 64))) return rc;
-      if ((rc = make_tmap_retiled(c, &L.tm_fc2_h, L.fc2_wt, (long long)g.d_inner * D / 64, 128))) return rc;
-#endif
-      if ((int)c->h_mlp.size() <= l) c->h_mlp.resize(l + 1);
-      bm::LayerConsts& hc = c->h_mlp[l];
-      CLM_CUDA(c, cudaMemcpy(hc.b_out, L.out_b, sizeof hc.b_out, cudaMemcpyDeviceToHost));
-      CLM_CUDA(c, cudaMemcpy(hc.b2, L.fc2_b, sizeof hc.b2, cudaMemcpyDeviceToHost));
-      CLM_CUDA(c, cudaMemcpy(hc.b1, b1f, sizeof hc.b1, cudaMemcpyDeviceToHost));
-    }
+    L.out_w32 = out_w; L.fc1_w32 = fc1_w; L.fc2_w32 = fc2_w;
+    if (l >= bm::MAX_LAYERS) return fail(c, CLM_ERR_INVALID, "n_layer > %d not supported by the fused block kernel", bm::MAX_LAYERS);
+    if ((rc = prepare_block_tail(c, l, 0))) return rc;
+    if ((int)c->h_mlp.size() <= l) c->h_mlp.resize(l + 1);
+    bm::LayerConsts& hc = c->h_mlp[l];
+    CLM_CUDA(c, cudaMemcpy(hc.b_out, L.out_b, sizeof hc.b_out, cudaMemcpyDeviceToHost));
+    CLM_CUDA(c, cudaMemcpy(hc.b2, L.fc2_b, sizeof hc.b2, cudaMemcpyDeviceToHost));
+    CLM_CUDA(c, cudaMemcpy(hc.b1, L.fc1_bf, sizeof hc.b1, cudaMemcpyDeviceToHost));
     // implicit filter k[l] = HyenaFilter.filter(Lmax)
     FilterGenParams fp{};
     const std::string Q = P + "mixer.filter_fn.";
@@ -1736,6 +1793,7 @@ int clm_predict_host(clm_ctx* c, const uint8_t* h_bases, const int64_t* h_offset
 int clm_gemm(clm_ctx* c, const void* d_A, const void* d_W, const float* d_bias, int M, int N, int K, int epi,
              void* d_out, const float* d_res, const float* d_w2, float b2, float* d_score, void* stream) {
   if (!c || !d_A || !d_W || !d_bias) return fail(c, CLM_ERR_INVALID, "clm_gemm: bad argument");
+  if (epi < EPI_BIAS_BF16 || epi > EPI_SCORE) return fail(c, CLM_ERR_INVALID, "gemm: unknown epilogue %d", epi);   // the tail-training epilogues are internal
   CUtensorMap tmB;
   int rc = make_tmap_bf16_2d(c, &tmB, d_W, (uint64_t)N, (uint64_t)K, epi == EPI_SCORE ? 256 : 128);
   if (rc) return rc;
@@ -2047,6 +2105,153 @@ float* head_live(clm_ctx* c, int i) {
   return it == c->w.end() ? nullptr : it->second.d;
 }
 
+// ---- the last block's tail (clm_tail_train_begin): its tensors in the order of the flat tail buffers
+enum { TT_OW, TT_OB, TT_G2, TT_B2, TT_W1, TT_B1, TT_W2, TT_B2F, TT_GF, TT_BF, kNumTailTensors };
+
+std::string tail_name(const clm_ctx* c, int i) {
+  static const char* sub[kNumTailTensors] = {"mixer.out_proj.weight", "mixer.out_proj.bias", "norm2.weight", "norm2.bias",
+                                             "mlp.fc1.weight", "mlp.fc1.bias", "mlp.fc2.weight", "mlp.fc2.bias", "", ""};
+  const std::string BB = "net.backbone.backbone.";
+  if (i == TT_GF) return BB + "ln_f.weight";
+  if (i == TT_BF) return BB + "ln_f.bias";
+  return BB + "layers." + std::to_string(c->cfg.n_layer - 1) + "." + sub[i];
+}
+
+long long tail_numel(const clm_ctx* c, int i) {
+  const long long D = c->cfg.d_model, DI = c->cfg.d_inner;
+  switch (i) {
+    case TT_OW: return D * D;
+    case TT_W1: case TT_W2: return DI * D;
+    case TT_B1: return DI;
+    default: return D;
+  }
+}
+
+long long tail_offset(const clm_ctx* c, int i) {
+  long long off = 0;
+  for (int k = 0; k < i; ++k) off += (tail_numel(c, k) + 63) / 64 * 64;
+  return off;
+}
+
+int tail_index(const clm_ctx* c, const char* name) {
+  std::string n(name ? name : "");
+  if (n.rfind("net.", 0) != 0) n = "net." + n;
+  for (int i = 0; i < kNumTailTensors; ++i)
+    if (n == tail_name(c, i)) return i;
+  return -1;
+}
+
+float* tail_live(clm_ctx* c, int i) {
+  auto it = c->w.find(tail_name(c, i));
+  return it == c->w.end() ? nullptr : it->second.d;
+}
+
+// split-K factor of tail_wgrad_kernel: about one CTA per SM over the output tiles, never more splits than token chunks
+int wgrad_splits(const clm_ctx* c, int O, int I, int n_chunks) {
+  const int tiles = (O / 128) * (I / 256);
+  return std::max(1, std::min(n_chunks, c->num_sms / tiles));
+}
+
+// C[o][i] = sum_t A[t][o] B[t][i] over M token rows (A [M,O], B [M,I] bf16, token-major) -> dW [O][I]
+int launch_wgrad(clm_ctx* c, const __nv_bfloat16* A, int O, const __nv_bfloat16* Bm, int I, int M, float* dW, cudaStream_t st) {
+  clm_ctx::TailTrain& t = c->tt;
+  if (int rc_attr = ensure_smem_attr(c, (const void*)(tail_wgrad_kernel), (int)(tw::SMEM_TOTAL))) return rc_attr;
+  CUtensorMap tmA, tmB;
+  int rc;
+  if ((rc = make_tmap_bf16_2d(c, &tmA, A, (uint64_t)M, (uint64_t)O, tw::KT))) return rc;
+  if ((rc = make_tmap_bf16_2d(c, &tmB, Bm, (uint64_t)M, (uint64_t)I, tw::KT))) return rc;
+  WgradParams wp{};
+  wp.part = t.wpart; wp.O = O; wp.I = I;
+  wp.n_chunks = (M + tw::KT - 1) / tw::KT;
+  const int splits = wgrad_splits(c, O, I, wp.n_chunks);
+  wp.chunks_per_split = (wp.n_chunks + splits - 1) / splits;
+  if ((long long)splits * O * I > t.wpart_elems) return fail(c, CLM_ERR_STATE, "wgrad: partials exceed their workspace");
+  tail_wgrad_kernel<<<dim3(I / 256, O / 128, splits), tw::THREADS, tw::SMEM_TOTAL, st>>>(tmA, tmB, wp);
+  CLM_LAUNCH_CHECK(c, "tail_wgrad");
+  const long long n = (long long)O * I;
+  wgrad_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(t.wpart, n, splits, dW);
+  CLM_LAUNCH_CHECK(c, "wgrad_reduce");
+  return 0;
+}
+
+// Recompute of the last block's tail from r0 (R) and y (Y), then its backward from the head's dz (score_bwd_kernel) and
+// dpooled, into the flat tail gradient buffer (csrc/tail_train.cuh for the formulas).
+int tail_backward(clm_ctx* c, int B, int T, cudaStream_t st) {
+  clm_ctx::TailTrain& t = c->tt;
+  const clm_config& g = c->cfg;
+  const int D = g.d_model, DI = g.d_inner, M = B * T, Tp = round_up(T, 128);
+  const int n_groups = (M + GEMM_BM - 1) / GEMM_BM * 4;
+  LayerW& L = c->layers[g.n_layer - 1];
+  float* G[kNumTailTensors];
+  for (int i = 0; i < kNumTailTensors; ++i) G[i] = t.grad + tail_offset(c, i);
+  int rc;
+  // ---- recompute: r1, LayerNorm2, fc1 (h and a kept), fc2 -> r2, ln_f statistics
+  transpose_ct_kernel<<<dim3((T + 63) / 64, D / 64, B), 256, 0, st>>>(c->Y, c->YT, T, Tp, D);
+  CLM_LAUNCH_CHECK(c, "transpose_ct");
+  GemmParams p{};
+  p.M = M; p.N = D; p.K = D; p.bias = L.out_b; p.out = t.R1; p.res = c->R; p.ldo = D; p.r32 = 1;
+  if ((rc = launch_gemm(c, c->YT, L.tm_out, p, EPI_BIAS_RES_F32, st))) return rc;
+  tail_ln_kernel<<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t.R1, L.ln2_g, L.ln2_b, t.n1, t.x2, t.rho1, M, g.layer_norm_eps);
+  CLM_LAUNCH_CHECK(c, "tail_ln2");
+  p = GemmParams{};
+  p.M = M; p.N = DI; p.K = D; p.bias = L.fc1_b; p.out = t.a; p.out2 = t.h; p.ldo = DI;
+  if ((rc = launch_gemm(c, t.x2, L.tm_fc1, p, EPI_BIAS_GELU_TANH_KEEP, st))) return rc;
+  p = GemmParams{};
+  p.M = M; p.N = D; p.K = DI; p.bias = L.fc2_b; p.out = t.R1; p.res = t.R1; p.ldo = D; p.r32 = 1;
+  if ((rc = launch_gemm(c, t.a, L.tm_fc2, p, EPI_BIAS_RES_F32, st))) return rc;
+  tail_ln_kernel<<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t.R1, nullptr, nullptr, t.n2, nullptr, t.rho2, M, g.layer_norm_eps);
+  CLM_LAUNCH_CHECK(c, "tail_ln_f");
+  // ---- K-major bf16 copies of W0, W2, W1 (the B operands of the dgrad GEMMs)
+  transpose_f32_bf16_kernel<<<dim3(D / 32, D / 32), 256, 0, st>>>(c->att0_w32, t.w0t, D, D);
+  transpose_f32_bf16_kernel<<<dim3(DI / 32, D / 32), 256, 0, st>>>(L.fc2_w32, t.w2t, D, DI);
+  transpose_f32_bf16_kernel<<<dim3(D / 32, DI / 32), 256, 0, st>>>(L.fc1_w32, t.w1t, DI, D);
+  CLM_LAUNCH_CHECK(c, "transpose_w");
+  // ---- dgrad: dr2 (with d ln_f, d fc2.bias), dh (d fc1.bias), dr1 (d norm2, d out_proj.bias)
+  p = GemmParams{};
+  p.M = M; p.N = D; p.K = D; p.out = t.dr2; p.ldo = D; p.nrm = t.n2; p.rho = t.rho2; p.gam = c->lnf_g;
+  p.score_in = c->score; p.rd = c->ht.rd; p.dp = c->ht.dpooled; p.T = T; p.colsum = t.colsum;
+  if ((rc = launch_gemm(c, t.dz, t.tm_w0t, p, EPI_TAIL_DHID, st))) return rc;
+  colsum_reduce_kernel<<<3 * D, 256, 0, st>>>(t.colsum, n_groups, 3, D, G[TT_GF], G[TT_BF], G[TT_B2F]);
+  CLM_LAUNCH_CHECK(c, "colsum_reduce");
+  p = GemmParams{};
+  p.M = M; p.N = DI; p.K = D; p.out = t.dh; p.ldo = DI; p.aux = t.h; p.colsum = t.colsum;
+  if ((rc = launch_gemm(c, t.dr2, t.tm_w2t, p, EPI_TAIL_DH, st))) return rc;
+  colsum_reduce_kernel<<<DI, 256, 0, st>>>(t.colsum, n_groups, 1, DI, G[TT_B1], nullptr, nullptr);
+  CLM_LAUNCH_CHECK(c, "colsum_reduce");
+  p = GemmParams{};
+  p.M = M; p.N = D; p.K = DI; p.out = t.dr1; p.ldo = D; p.nrm = t.n1; p.rho = t.rho1; p.gam = L.ln2_g; p.aux = t.dr2;
+  p.colsum = t.colsum;
+  if ((rc = launch_gemm(c, t.dh, t.tm_w1t, p, EPI_TAIL_DR1, st))) return rc;
+  colsum_reduce_kernel<<<3 * D, 256, 0, st>>>(t.colsum, n_groups, 3, D, G[TT_G2], G[TT_B2], G[TT_OB]);
+  CLM_LAUNCH_CHECK(c, "colsum_reduce");
+  // ---- wgrad: fc2, fc1, out_proj
+  if ((rc = launch_wgrad(c, t.dr2, D, t.a, DI, M, G[TT_W2], st))) return rc;
+  if ((rc = launch_wgrad(c, t.dh, DI, t.x2, D, M, G[TT_W1], st))) return rc;
+  if ((rc = launch_wgrad(c, t.dr1, D, c->YT, D, M, G[TT_OW], st))) return rc;
+  return 0;
+}
+
+
+// After the tail's AdamW update: the live fp32 tensors, what the forward derives from them (prepare_block_tail) and the
+// block-tail constants of the last layer, written into the device copy and from there into the constant bank.
+int tail_refresh(clm_ctx* c, cudaStream_t st) {
+  clm_ctx::TailTrain& t = c->tt;
+  const int l = c->cfg.n_layer - 1, D = c->cfg.d_model, DI = c->cfg.d_inner;
+  for (int i = 0; i < kNumTailTensors; ++i)
+    CLM_CUDA(c, cudaMemcpyAsync(tail_live(c, i), t.param + tail_offset(c, i), (size_t)tail_numel(c, i) * sizeof(float),
+                                cudaMemcpyDeviceToDevice, st));
+  int rc;
+  if ((rc = prepare_block_tail(c, l, st))) return rc;
+  const LayerW& L = c->layers[l];
+  bm::LayerConsts* dc = t.d_consts + l;
+  CLM_CUDA(c, cudaMemcpyAsync(dc->b_out, L.out_b, D * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CLM_CUDA(c, cudaMemcpyAsync(dc->b2, L.fc2_b, D * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CLM_CUDA(c, cudaMemcpyAsync(dc->b1, L.fc1_bf, DI * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CLM_CUDA(c, cudaMemcpyToSymbolAsync(bm::c_mlp, t.d_consts, c->h_mlp.size() * sizeof(bm::LayerConsts), 0, cudaMemcpyDeviceToDevice, st));
+  g_const_owner[c->device & 63] = c;
+  return 0;
+}
+
 }  // namespace
 
 int clm_head_train_begin(clm_ctx* c, const clm_head_train_cfg* cfg) {
@@ -2108,6 +2313,13 @@ int clm_head_train_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int
   // score_pool_kernel and pooled from head_fused_kernel
   if (!c->fused_mlp || !c->fused_score_pool || !c->fused_head || c->dbg_layer >= 0)
     return fail(c, CLM_ERR_STATE, "clm_head_train_step needs the fused forward (options fused_mlp, fused_score_pool, fused_head on, no debug stop)");
+  if (c->tt.on) {   // the tail's backward recomputes from block L's input residual, which only survives in R without its store
+    if (!c->skip_dead_res)
+      return fail(c, CLM_ERR_STATE, "clm_head_train_step with the tail in training needs option skip_dead_res on (r0 must survive in R)");
+    if ((long long)B * T > c->tt.max_tokens)
+      return fail(c, CLM_ERR_STATE, "clm_head_train_step: batch of %lld tokens exceeds the %lld sized by clm_tail_train_begin",
+                  (long long)B * T, c->tt.max_tokens);
+  }
   cudaStream_t st = (cudaStream_t)stream;
   int rc = clm_forward(c, d_ids, ids_dtype, B, T, h.fwd_logits, nullptr, st);
   if (rc) return rc;
@@ -2166,12 +2378,14 @@ int clm_head_train_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int
     sp.b0f = c->att0_bf; sp.w2 = c->att2_w; sp.score = c->score; sp.rd = h.rd; sp.gdp = h.gdp;
     sp.part_dw = h.part_dw; sp.part_vec = h.part_vec;
     sp.B = B; sp.T = T; sp.tiles_per_seq = tiles_per_seq; sp.num_tiles = B * tiles_per_seq;
+    sp.dz_out = c->tt.on ? c->tt.dz : nullptr;
     const int grid = 2 * std::min(sp.num_tiles, h.n_cta / 2);
     score_bwd_kernel<<<grid, sb::THREADS, sb::SMEM_TOTAL, st>>>(tmX, tmW, sp);
     CLM_LAUNCH_CHECK(c, "score_bwd");
     score_bwd_reduce_kernel<<<D, 256, 0, st>>>(h.part_dw, h.part_vec, grid, c->lnf_g, c->lnf_b, G[HT_A0W], G[HT_A0B], G[HT_A2W], G[HT_A2B]);
     CLM_LAUNCH_CHECK(c, "score_bwd_reduce");
   }
+  if (c->tt.on && (rc = tail_backward(c, B, T, st))) return rc;
   // ---- AdamW on the master copies, then refresh what the forward reads
   AdamWParams ap{};
   ap.p = h.param; ap.m = h.m; ap.v = h.v; ap.g = h.grad; ap.n = h.n;
@@ -2179,11 +2393,17 @@ int clm_head_train_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int
   ap.step = h.step; ap.status = status;
   adamw_kernel<<<(unsigned)std::min<long long>((h.n + 255) / 256, 4LL * c->num_sms), 256, 0, st>>>(ap);
   CLM_LAUNCH_CHECK(c, "adamw");
+  if (c->tt.on) {   // same hyper-parameters, step counter and skip rule; its own learning rate
+    ap.p = c->tt.param; ap.m = c->tt.m; ap.v = c->tt.v; ap.g = c->tt.grad; ap.n = c->tt.n; ap.lr = c->tt.lr;
+    adamw_kernel<<<(unsigned)std::min<long long>((c->tt.n + 255) / 256, 4LL * c->num_sms), 256, 0, st>>>(ap);
+    CLM_LAUNCH_CHECK(c, "adamw");
+  }
   adamw_step_kernel<<<1, 1, 0, st>>>(h.step, status);
   CLM_LAUNCH_CHECK(c, "adamw_step");
   for (int i = 0; i < kNumHeadTensors; ++i)
     CLM_CUDA(c, cudaMemcpyAsync(head_live(c, i), h.param + head_offset(i), (size_t)kHeadTensors[i].numel * sizeof(float),
                                 cudaMemcpyDeviceToDevice, st));
+  if (c->tt.on && (rc = tail_refresh(c, st))) return rc;
   if ((rc = refresh_scorer(c, st))) return rc;
   ++h.calls;
   return 0;
@@ -2192,8 +2412,14 @@ int clm_head_train_step(clm_ctx* c, const void* d_ids, int ids_dtype, int B, int
 int clm_head_grad_copy(clm_ctx* c, const char* name, float* d_dst, void* stream) {
   if (!c || !name || !d_dst) return fail(c, CLM_ERR_INVALID, "clm_head_grad_copy: bad argument");
   if (!c->ht.on) return fail(c, CLM_ERR_STATE, "clm_head_grad_copy before clm_head_train_begin");
+  if (const int k = tail_index(c, name); k >= 0) {
+    if (!c->tt.on) return fail(c, CLM_ERR_STATE, "clm_head_grad_copy('%s') before clm_tail_train_begin", name);
+    CLM_CUDA(c, cudaMemcpyAsync(d_dst, c->tt.grad + tail_offset(c, k), (size_t)tail_numel(c, k) * sizeof(float),
+                                cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return 0;
+  }
   const int i = head_index(name);
-  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_grad_copy: '%s' is not a trainable head tensor", name);
+  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_grad_copy: '%s' is not a trainable head or tail tensor", name);
   CLM_CUDA(c, cudaMemcpyAsync(d_dst, c->ht.grad + head_offset(i), (size_t)kHeadTensors[i].numel * sizeof(float),
                               cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
@@ -2202,8 +2428,18 @@ int clm_head_grad_copy(clm_ctx* c, const char* name, float* d_dst, void* stream)
 int clm_head_export(clm_ctx* c, const char* name, float* h_dst) {
   if (!c || !name || !h_dst) return fail(c, CLM_ERR_INVALID, "clm_head_export: bad argument");
   if (!c->finalized) return fail(c, CLM_ERR_STATE, "clm_head_export before clm_finalize");
+  if (const int k = tail_index(c, name); k >= 0) {
+    CLM_CUDA(c, cudaSetDevice(c->device));
+    CLM_CUDA(c, cudaDeviceSynchronize());
+    const float* src = c->tt.on ? c->tt.param + tail_offset(c, k) : tail_live(c, k);
+    if (!src) return fail(c, CLM_ERR_MISSING, "clm_head_export: weight '%s' was not loaded", name);
+    CLM_CUDA(c, cudaMemcpy(h_dst, src, (size_t)tail_numel(c, k) * sizeof(float), cudaMemcpyDeviceToHost));
+    if (c->tt.on)   // the host copy of the block-tail constants follows the trained ones
+      CLM_CUDA(c, cudaMemcpy(c->h_mlp.data(), c->tt.d_consts, c->h_mlp.size() * sizeof(bm::LayerConsts), cudaMemcpyDeviceToHost));
+    return 0;
+  }
   const int i = head_index(name);
-  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_export: '%s' is not a head tensor", name);
+  if (i < 0) return fail(c, CLM_ERR_INVALID, "clm_head_export: '%s' is not a head or tail tensor", name);
   CLM_CUDA(c, cudaSetDevice(c->device));
   CLM_CUDA(c, cudaDeviceSynchronize());
   const float* src = c->ht.on ? c->ht.param + head_offset(i) : head_live(c, i);
@@ -2211,6 +2447,56 @@ int clm_head_export(clm_ctx* c, const char* name, float* h_dst) {
   CLM_CUDA(c, cudaMemcpy(h_dst, src, (size_t)kHeadTensors[i].numel * sizeof(float), cudaMemcpyDeviceToHost));
   if (c->ht.on)
     CLM_CUDA(c, cudaMemcpy(&c->att2_b, c->ht.param + head_offset(HT_A2B), sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int clm_tail_train_begin(clm_ctx* c, float lr) {
+  if (!c) return CLM_ERR_INVALID;
+  if (!c->ht.on) return fail(c, CLM_ERR_STATE, "clm_tail_train_begin before clm_head_train_begin");
+  if (c->tt.on) return fail(c, CLM_ERR_STATE, "clm_tail_train_begin: the tail is already in training on this context");
+  if (c->ht.calls > 0) return fail(c, CLM_ERR_STATE, "clm_tail_train_begin after a clm_head_train_step: call it before the first step");
+  if (!(lr >= 0.f)) return fail(c, CLM_ERR_INVALID, "clm_tail_train_begin: lr >= 0");
+  const clm_config& g = c->cfg;
+  if (g.n_layer < 1 || g.d_model != 256 || g.d_inner != 1024)
+    return fail(c, CLM_ERR_INVALID, "clm_tail_train_begin: needs d_model 256 and d_inner 1024 (the fused block tail's shapes)");
+  for (int i = 0; i < kNumTailTensors; ++i)
+    if (!tail_live(c, i)) return fail(c, CLM_ERR_MISSING, "clm_tail_train_begin: weight '%s' was not loaded", tail_name(c, i).c_str());
+  CLM_CUDA(c, cudaSetDevice(c->device));
+  clm_ctx::TailTrain& t = c->tt;
+  const size_t M = (size_t)c->max_tokens, D = g.d_model, DI = g.d_inner;
+  const size_t n_groups = (M + GEMM_BM - 1) / GEMM_BM * 4;
+  t.n = tail_offset(c, kNumTailTensors);
+  int rc;
+  for (float** p : {&t.param, &t.grad, &t.m, &t.v})
+    if ((rc = dev_alloc(c, p, (size_t)t.n))) return rc;
+  if ((rc = dev_alloc(c, &t.d_consts, c->h_mlp.size()))) return rc;
+  if ((rc = dev_alloc(c, &t.R1, (M + 160) * D))) return rc;
+  for (float** p : {&t.rho1, &t.rho2})
+    if ((rc = dev_alloc(c, p, M))) return rc;
+  for (__nv_bfloat16** p : {&t.n1, &t.x2, &t.n2, &t.dz, &t.dr2, &t.dr1})
+    if ((rc = dev_alloc(c, p, M * D))) return rc;
+  for (__nv_bfloat16** p : {&t.h, &t.a, &t.dh})
+    if ((rc = dev_alloc(c, p, M * DI))) return rc;
+  if ((rc = dev_alloc(c, &t.w0t, D * D))) return rc;
+  if ((rc = dev_alloc(c, &t.w2t, DI * D))) return rc;
+  if ((rc = dev_alloc(c, &t.w1t, D * DI))) return rc;
+  if ((rc = dev_alloc(c, &t.colsum, n_groups * std::max(3 * D, DI)))) return rc;
+  t.wpart_elems = (long long)std::max(c->num_sms, 8) * 128 * 256;   // wgrad_splits keeps splits x tiles <= max(num_sms, tiles)
+  if ((rc = dev_alloc(c, &t.wpart, (size_t)t.wpart_elems))) return rc;
+  if ((rc = make_tmap_bf16_2d(c, &t.tm_w0t, t.w0t, D, D, 256))) return rc;
+  if ((rc = make_tmap_bf16_2d(c, &t.tm_w2t, t.w2t, DI, D, 128))) return rc;
+  if ((rc = make_tmap_bf16_2d(c, &t.tm_w1t, t.w1t, D, DI, 256))) return rc;
+  CLM_CUDA(c, cudaMemset(t.param, 0, (size_t)t.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(t.grad, 0, (size_t)t.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(t.m, 0, (size_t)t.n * sizeof(float)));
+  CLM_CUDA(c, cudaMemset(t.v, 0, (size_t)t.n * sizeof(float)));
+  for (int i = 0; i < kNumTailTensors; ++i)
+    CLM_CUDA(c, cudaMemcpy(t.param + tail_offset(c, i), tail_live(c, i), (size_t)tail_numel(c, i) * sizeof(float), cudaMemcpyDeviceToDevice));
+  CLM_CUDA(c, cudaMemcpy(t.d_consts, c->h_mlp.data(), c->h_mlp.size() * sizeof(bm::LayerConsts), cudaMemcpyHostToDevice));
+  CLM_CUDA(c, cudaDeviceSynchronize());
+  t.lr = lr;
+  t.max_tokens = (long long)M;
+  t.on = true;
   return 0;
 }
 

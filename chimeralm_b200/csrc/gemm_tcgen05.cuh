@@ -25,6 +25,11 @@ enum GemmEpilogue : int {
   EPI_BIAS_GELU_TANH = 1,  // out_bf16 = gelu_tanh(acc + bias)          (HyenaMlp fc1, A.6)
   EPI_BIAS_RES_F32 = 2,    // out_f32  = acc + bias + res               (out_proj / fc2 + residual)
   EPI_SCORE = 3,           // score[m] = sum_n gelu_erf(acc + bias)[n] * w2[n] + b2   (needs BN == N)
+  EPI_BIAS_GELU_TANH_KEEP = 4,   // EPI_BIAS_GELU_TANH, and out2_bf16 = acc + bias      (the tail's fc1 recompute)
+  // dgrad GEMMs of the last block's tail (csrc/tail_train.cuh, gemm_tail_epilogue): bf16 out, per-warp column sums
+  EPI_TAIL_DHID = 5,       // dz . W0 + w_t dp -> ln_f backward -> dr2                  (needs BN == N == 256)
+  EPI_TAIL_DH = 6,         // dr2 . W2 -> * gelu_tanh'(h) -> dh
+  EPI_TAIL_DR1 = 7,        // dh . W1 -> norm2 backward + dr2 -> dr1                    (needs BN == N == 256)
 };
 
 struct GemmParams {
@@ -37,7 +42,21 @@ struct GemmParams {
   float* score;        // EPI_SCORE: [M]
   long long ldo;
   int r32;             // EPI_BIAS_RES_F32: res/out use the R32 blocked layout (N must be 256)
+  void* out2;          // EPI_BIAS_GELU_TANH_KEEP: bf16 [M,ldo] pre-activation
+  // EPI_TAIL_*
+  const __nv_bfloat16* nrm;   // DHID: n2, DR1: n1 (bf16 [M,256])
+  const float* rho;           // DHID: rho2, DR1: rho1 ([M])
+  const float* gam;           // DHID: ln_f.weight, DR1: norm2.weight
+  const __nv_bfloat16* aux;   // DH: h (bf16 [M,ldo]), DR1: dr2 (bf16 [M,256])
+  const float* score_in;      // DHID: the forward's scores [M]
+  const float* rd;            // DHID: per read (softmax max, 1 / normaliser, -, -)
+  const float* dp;            // DHID: dpooled [B,256]
+  int T;                      // DHID: tokens per read (row = b * T + t)
+  float* colsum;              // per-warp column partials [(M / 128) * 4][3 or 1][N]
 };
+
+template <int BN, int EPI>
+__device__ void gemm_tail_epilogue(const GemmParams& p, uint32_t tmem_base, int m0, int n0, int q, int lane);   // tail_train.cuh
 
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_BK = 64;   // 64 bf16 = 128 bytes = one swizzle row
@@ -157,6 +176,11 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       }
       ptx::umma_commit(tmem_full_bar);
     }
+  } else if constexpr (EPI >= EPI_TAIL_DHID) {
+    ptx::mbar_wait(tmem_full_bar, 0);
+    ptx::tc_fence_after_sync();
+    gemm_tail_epilogue<BN, EPI>(p, tmem_base, m0, n0, warp & 3, lane);
+    ptx::tc_fence_before_sync();
   } else {
     // ---------------- epilogue: warps 2..5, TMEM lane quarter = warp % 4
     const int q = warp & 3;
@@ -180,8 +204,17 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         v[j + 2] = __uint_as_float(r[j + 2]) + b4.z;
         v[j + 3] = __uint_as_float(r[j + 3]) + b4.w;
       }
-      if constexpr (EPI == EPI_BIAS_BF16 || EPI == EPI_BIAS_GELU_TANH) {
-        if constexpr (EPI == EPI_BIAS_GELU_TANH) {
+      if constexpr (EPI == EPI_BIAS_BF16 || EPI == EPI_BIAS_GELU_TANH || EPI == EPI_BIAS_GELU_TANH_KEEP) {
+        if constexpr (EPI == EPI_BIAS_GELU_TANH_KEEP) {
+          if (row_ok) {
+            uint4* o2 = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.out2) + row * p.ldo + n);
+#pragma unroll
+            for (int j = 0; j < 32; j += 8)
+              o2[j / 8] = make_uint4(pack_bf16(v[j], v[j + 1]), pack_bf16(v[j + 2], v[j + 3]), pack_bf16(v[j + 4], v[j + 5]),
+                                     pack_bf16(v[j + 6], v[j + 7]));
+          }
+        }
+        if constexpr (EPI == EPI_BIAS_GELU_TANH || EPI == EPI_BIAS_GELU_TANH_KEEP) {
 #pragma unroll
           for (int j = 0; j < 32; ++j) v[j] = gelu_tanh_f(v[j]);
         }

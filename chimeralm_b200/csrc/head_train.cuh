@@ -242,6 +242,7 @@ struct ScoreBwdParams {
   float* part_dw;      // [grid][128][256]
   float* part_vec;     // [grid][3][128]: sum dz, sum ds a, (sum ds, 0, ...)
   int B, T, tiles_per_seq, num_tiles;
+  __nv_bfloat16* dz_out;   // null, or [B*T][256]: this CTA's half of dz as bf16 (training the last block's tail)
 };
 
 namespace sb {
@@ -419,6 +420,11 @@ score_bwd_kernel(const __grid_constant__ CUtensorMap tmXN, const __grid_constant
           const int chunk = (ci & 1) * 4 + c8;
           *reinterpret_cast<uint4*>(dzrow + ((chunk ^ (r & 7)) << 4)) =
               make_uint4(pk[4 * c8], pk[4 * c8 + 1], pk[4 * c8 + 2], pk[4 * c8 + 3]);
+        }
+        if (p.dz_out && r < valid) {
+          uint4* g = reinterpret_cast<uint4*>(p.dz_out + ((long long)b * p.T + t0 + r) * 256 + half * HALF + ci * 32);
+#pragma unroll
+          for (int c8 = 0; c8 < 4; ++c8) g[c8] = make_uint4(pk[4 * c8], pk[4 * c8 + 1], pk[4 * c8 + 2], pk[4 * c8 + 3]);
         }
         acc_dz[ci] += warp_reduce_scatter32(vz, lane);
         acc_da[ci] += warp_reduce_scatter32(va, lane);

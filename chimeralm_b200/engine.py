@@ -14,7 +14,7 @@ import torch
 
 from . import _lib
 from .config import DEFAULT_CONFIG, HyenaConfig
-from .weights import HEAD_PREFIX
+from .weights import BACKBONE_PREFIX, HEAD_PREFIX
 
 _IDS_DTYPES = {torch.uint8: _lib.CLM_U8, torch.int32: _lib.CLM_I32, torch.int64: _lib.CLM_I64}
 
@@ -24,6 +24,14 @@ def _full_name(name: str) -> str:
     if name.startswith("net."):
         return name
     return "net." + name if name.startswith("head.") else HEAD_PREFIX + name
+
+
+def tail_keys(n_layer: int) -> list[str]:
+    """State-dict keys of the last block's tail and ln_f, the tensors `Engine.tail_train_begin` adds to training."""
+    p = f"{BACKBONE_PREFIX}layers.{n_layer - 1}."
+    return [p + "mixer.out_proj.weight", p + "mixer.out_proj.bias", p + "norm2.weight", p + "norm2.bias",
+            p + "mlp.fc1.weight", p + "mlp.fc1.bias", p + "mlp.fc2.weight", p + "mlp.fc2.bias",
+            BACKBONE_PREFIX + "ln_f.weight", BACKBONE_PREFIX + "ln_f.bias"]
 
 
 def _stream_ptr(device) -> C.c_void_p:
@@ -87,11 +95,15 @@ class Engine:
 
     def load_state_dict(self, sd) -> None:
         self._head_shapes = getattr(self, "_head_shapes", {})
+        self._tail_shapes = getattr(self, "_tail_shapes", {})
+        tail = set(tail_keys(self.cfg.n_layer))
         for name, t in sd.items():
             if not name.startswith("net."):
                 name = "net." + name
             if name.startswith(HEAD_PREFIX):
                 self._head_shapes[name] = tuple(t.shape)
+            if name in tail:
+                self._tail_shapes[name] = tuple(t.shape)
             a = t.detach().to(torch.float32).cpu().contiguous().numpy()
             shape = (C.c_int64 * max(a.ndim, 1))(*a.shape) if a.ndim else (C.c_int64 * 1)(1)
             rc = self.lib.clm_load_tensor(self.ctx, name.encode(), a.ctypes.data_as(C.c_void_p), _lib.CLM_F32,
@@ -272,17 +284,28 @@ class Engine:
                     self.set_option("tc_conv", 1)
         return loss
 
+    def tail_train_begin(self, lr: float) -> None:
+        """Train the last block's tail (out_proj, norm2, fc1, fc2) and ln_f together with the head from the next step on,
+        with learning rate `lr` and the head's other AdamW settings (clm_tail_train_begin).  Call after
+        `head_train_begin` and before the first `head_train_step`."""
+        self._check(self.lib.clm_tail_train_begin(self.ctx, float(lr)), "clm_tail_train_begin")
+
+    def _shape(self, name: str):
+        name = _full_name(name)
+        return self._tail_shapes[name] if name in self._tail_shapes else self._head_shapes[name]
+
     def head_grad(self, name: str) -> torch.Tensor:
-        """Gradient of head tensor `name` (state-dict key) from the last training step, float32 on this device."""
-        numel = int(np.prod(self._head_shapes[_full_name(name)]))
-        out = torch.empty(numel, dtype=torch.float32, device=self.device)
+        """Gradient of head or tail tensor `name` (state-dict key; tail keys in full) from the last training step,
+        float32 on this device."""
+        shape = self._shape(name)
+        out = torch.empty(int(np.prod(shape)), dtype=torch.float32, device=self.device)
         self._check(self.lib.clm_head_grad_copy(self.ctx, _full_name(name).encode(), C.c_void_p(out.data_ptr()),
                                                 _stream_ptr(self.device)), "clm_head_grad_copy")
-        return out.view(self._head_shapes[_full_name(name)])
+        return out.view(shape)
 
     def head_export(self, name: str) -> torch.Tensor:
-        """Current value of head tensor `name` as a CPU float32 tensor (synchronises the device)."""
-        shape = self._head_shapes[_full_name(name)]
+        """Current value of head or tail tensor `name` as a CPU float32 tensor (synchronises the device)."""
+        shape = self._shape(name)
         out = torch.empty(shape, dtype=torch.float32)
         self._check(self.lib.clm_head_export(self.ctx, _full_name(name).encode(), C.c_void_p(out.data_ptr())),
                     "clm_head_export")
@@ -291,6 +314,11 @@ class Engine:
     def head_state_dict(self) -> dict:
         """Every trainable head tensor under its state-dict name."""
         return {k: self.head_export(k) for k in self._head_shapes}
+
+    def tail_state_dict(self) -> dict:
+        """The ten tensors of the last block's tail and ln_f under their state-dict names (their loaded values when the
+        tail is not in training)."""
+        return {k: self.head_export(k) for k in tail_keys(self.cfg.n_layer)}
 
     # ------------------------------------------------------------------ evaluation on labelled reads
     def eval_step(self, input_ids: torch.Tensor, targets: torch.Tensor, check: bool = True):

@@ -212,7 +212,7 @@ def evaluate(engine, seqs, labels, batch_size: int = 32):
 @dataclass
 class Validation:
     """Validation of a training run: `records[k]` holds the metrics after epoch k (0 = before training), `best` the
-    chosen epoch and `head` the head's tensors after it."""
+    chosen epoch and `head` the trained tensors after it (the head's, and with `train_tail` the tail's too)."""
     records: list
     best: int
     head: dict
@@ -252,10 +252,20 @@ def _validate(engine, val, batch_size, epoch, train_loss) -> dict:
     return rec
 
 
+def trained_state_dict(engine, train_tail: bool) -> dict:
+    """The tensors a run trains, as they stand: the head's, and with `train_tail` the last block's tail and ln_f."""
+    out = dict(engine.head_state_dict())
+    if train_tail:
+        out.update(engine.tail_state_dict())
+    return out
+
+
 def fit(engine, seqs, labels, *, epochs: int = 3, batch_size: int = 32, seed: int = 0, lr: float = 1e-3,
-        weight_decay: float = 0.01, dropout: float = 0.1, log_every: int = 0, val=None, patience: int | None = None):
+        weight_decay: float = 0.01, dropout: float = 0.1, log_every: int = 0, val=None, patience: int | None = None,
+        train_tail: bool = False, tail_lr: float | None = None):
     """Train the head of `engine` on (seqs, labels): per epoch the length-bucketed batches run in an order shuffled by
-    `seed` and the epoch.  Returns the mean loss of every epoch.
+    `seed` and the epoch.  Returns the mean loss of every epoch.  With `train_tail` the last block's tail (out_proj,
+    norm2, fc1, fc2) and ln_f train together with the head, with learning rate `tail_lr` (default `lr`).
 
     With `val` = (seqs, labels) of held-out reads the head is evaluated (`evaluate`, dropout off) before training
     (epoch 0, reported only) and after every epoch, and `patience` stops training after that many epochs without a
@@ -263,6 +273,8 @@ def fit(engine, seqs, labels, *, epochs: int = 3, batch_size: int = 32, seed: in
     (`best_epoch`) and the head's tensors after it."""
     if val is not None and epochs < 1:
         raise ValueError("validation needs at least one epoch")
+    if tail_lr is not None and not train_tail:
+        raise ValueError("tail_lr needs train_tail")
     labels = np.asarray(labels, np.int64)
     lens = np.array([len(s) for s in seqs], np.int64)
     batches = make_batches(lens, batch_size)
@@ -270,6 +282,8 @@ def fit(engine, seqs, labels, *, epochs: int = 3, batch_size: int = 32, seed: in
     max_t = max(int(lens[b].max()) + 1 for b in batches)
     engine.reserve(max_b, max_t, max(len(b) * (int(lens[b].max()) + 1) for b in batches))
     engine.head_train_begin(lr=lr, weight_decay=weight_decay, dropout=dropout, seed=seed)
+    if train_tail:
+        engine.tail_train_begin(lr if tail_lr is None else tail_lr)
     history = []
     if val is not None:
         run = Validation([], 0, {}, False)
@@ -289,7 +303,7 @@ def fit(engine, seqs, labels, *, epochs: int = 3, batch_size: int = 32, seed: in
         if val is not None:
             # the export also refreshes the forward's copy of attention.2.bias, so that the validation forward is the
             # forward of the saved checkpoint bit for bit
-            head = engine.head_state_dict()
+            head = trained_state_dict(engine, train_tail)
             run.records.append(_validate(engine, val, batch_size, ep + 1, history[-1]))
             if best_epoch(run.records) == ep + 1:
                 run.best, run.head = ep + 1, head
@@ -304,9 +318,10 @@ def fit(engine, seqs, labels, *, epochs: int = 3, batch_size: int = 32, seed: in
     return history, run
 
 
-def tuned_state_dict(base_sd, engine) -> "OrderedDict[str, torch.Tensor]":
-    """`base_sd` with its head tensors replaced by the engine's trained ones; every other tensor is the input's own."""
-    return with_head(base_sd, engine.head_state_dict())
+def tuned_state_dict(base_sd, engine, train_tail: bool = False) -> "OrderedDict[str, torch.Tensor]":
+    """`base_sd` with its head tensors (and with `train_tail` the tail's) replaced by the engine's trained ones; every
+    other tensor is the input's own."""
+    return with_head(base_sd, trained_state_dict(engine, train_tail))
 
 
 def with_head(base_sd, head) -> "OrderedDict[str, torch.Tensor]":
@@ -319,16 +334,20 @@ def with_head(base_sd, head) -> "OrderedDict[str, torch.Tensor]":
 
 def finetune(data_path, ckpt_path, output_path, *, epochs: int = 3, lr: float = 1e-3, batch_size: int = 32,
              seed: int = 0, seed_weights: int = 0, device: int = 0, weight_decay: float = 0.01,
-             dropout: float = 0.1, val_path=None, patience: int | None = None) -> list[float]:
+             dropout: float = 0.1, val_path=None, patience: int | None = None, train_tail: bool = False,
+             tail_lr: float | None = None) -> list[float]:
     """The `finetune` command: labelled reads -> trained head -> Lightning-layout checkpoint at `output_path`.
+    With `train_tail` the last block's tail and ln_f train too (`fit`), and the checkpoint replaces those tensors as well.
 
     With `val_path` (labelled reads, `read_labelled`) the head is validated before training and after every epoch
     (`fit`); the checkpoint holds the head of the chosen epoch (`best_epoch`), and the records go to
     `<output_path>.val.json`.  `patience` (needs `val_path`) stops after that many epochs without a better F1."""
-    from .engine import Engine
+    from .engine import Engine, tail_keys
 
     if patience is not None and (val_path is None or patience < 1):
         raise ValueError("patience needs validation reads (--val) and must be >= 1")
+    if tail_lr is not None and not train_tail:
+        raise ValueError("--tail-lr needs --train-tail")
     sd = load_checkpoint(ckpt_path) if ckpt_path is not None else make_state_dict(seed_weights)
     if not any(k.startswith(BACKBONE_PREFIX) for k in sd):
         raise ValueError("the checkpoint holds no backbone tensors (net.backbone.backbone.*)")
@@ -343,15 +362,18 @@ def finetune(data_path, ckpt_path, output_path, *, epochs: int = 3, lr: float = 
     try:
         if val is None:
             history = fit(eng, seqs, labels, epochs=epochs, batch_size=batch_size, seed=seed, lr=lr,
-                          weight_decay=weight_decay, dropout=dropout)
-            out = tuned_state_dict(sd, eng)
+                          weight_decay=weight_decay, dropout=dropout, train_tail=train_tail, tail_lr=tail_lr)
+            out = tuned_state_dict(sd, eng, train_tail)
         else:
             history, run = fit(eng, seqs, labels, epochs=epochs, batch_size=batch_size, seed=seed, lr=lr,
-                               weight_decay=weight_decay, dropout=dropout, val=val, patience=patience)
+                               weight_decay=weight_decay, dropout=dropout, val=val, patience=patience,
+                               train_tail=train_tail, tail_lr=tail_lr)
             out = with_head(sd, run.head)
+        tail = set(tail_keys(eng.cfg.n_layer)) if train_tail else set()
     finally:
         eng.close()
-    assert all(torch.equal(out[k], sd[k]) for k in sd if not k.startswith(HEAD_PREFIX))
+    # every tensor that was not trained equals the input
+    assert all(torch.equal(out[k], sd[k]) for k in sd if not (k.startswith(HEAD_PREFIX) or k in tail))
     Path(output_path).parent.mkdir(parents=True, exist_ok=True)
     save_lightning_ckpt(out, output_path)
     if val is not None:

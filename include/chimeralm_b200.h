@@ -238,6 +238,24 @@ int clm_head_grad_copy(clm_ctx* ctx, const char* name, float* d_dst, void* strea
  * changes no logit, attention weight or label. */
 int clm_head_export(clm_ctx* ctx, const char* name, float* h_dst);
 
+/* ---- Fine-tuning of the last block's tail together with the head ----------------------------
+ * Opt-in widening of the trainable set by the tail of the last block (layer L = n_layer - 1: mixer.out_proj, the residual,
+ * norm2, mlp.fc1, GELU-tanh, mlp.fc2, the residual) and ln_f: ten tensors, 592 384 parameters,
+ *   net.backbone.backbone.layers.L.mixer.out_proj.{weight,bias}, ...layers.L.norm2.{weight,bias},
+ *   ...layers.L.mlp.fc1.{weight,bias}, ...layers.L.mlp.fc2.{weight,bias}, net.backbone.backbone.ln_f.{weight,bias}.
+ * Everything upstream (embedding, blocks 0..L-1, block L's mixer up to the long convolution, filters, spectrum tables, the
+ * tensor-core range factors) stays bit-identical.  The tail trains with the head's AdamW hyper-parameters, step counter and
+ * skip-on-bad-status rule, with its own learning rate `lr`; no dropout inside the backbone.
+ * Call after clm_head_train_begin and before the first clm_head_train_step; from then on every clm_head_train_step also
+ * trains the tail (its signature and the head's gradients are unchanged), and after each step the forward reads the
+ * updated tail.  Allocates the tail's master copies, AdamW state and every buffer the tail's backward needs, for batches of
+ * up to the token budget of the last clm_reserve (about 11.5 KB per token); a step allocates nothing.  The step needs
+ * option skip_dead_res on (block L's input residual must survive the forward).  A second call, a call after a step or a
+ * call without head training returns CLM_ERR_STATE.  clm_head_grad_copy and clm_head_export accept the ten tail keys
+ * (full state-dict names); export returns the loaded value when the tail is not in training.  Without this call the
+ * library behaves exactly as without it. */
+int clm_tail_train_begin(clm_ctx* ctx, float lr);
+
 /* ---- Evaluation on labelled reads ------------------------------------------------------------
  * Replaces the loss half of ClassificationLit.validation_step / test_step, i.e. model_step without an optimizer step
  * (cross-entropy on net(input_ids), chimeralm/models/basic_module.py:87-104): clm_forward exactly as above (same logits,
